@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (this repo's CUDA path)
   python bench.py --impl reference --gpus N --steps K ...   (CPU arm: the reference's path)
+  ... --dump-outputs DIR    also write obs / reward / done of the last timed step as DIR/<name>.npy (rank 0)
 
 Workload (BASELINE.json configs[1]): Solo12, task walk, torque control, num_history_stack 1,
 frame_skip 4 at 1/240 s, 4096 envs per GPU, random actions U(-1,1)^12, auto-reset on.
@@ -46,6 +47,25 @@ def workload_config(n, world):
                       "arm, looked up in the bit-identical reset cache by the GPU arm",
             "l2": "GPU arm: flushed (256 MiB write) between timed steps, per-step CUDA events summed; CPU arm: not applicable",
             "parallelism": f"env-shard x{world}"}
+
+
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(path, arrays):
+    """Write what the timed path returned in its last step as `path/<name>.npy`, float32, so that two builds can be
+    compared output for output.  Above 64 MiB in all, the same fixed, seeded sample of rows (envs) is kept in every
+    array."""
+    arrays = {k: np.asarray(v, dtype=np.float32) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a.nbytes for a in arrays.values()) // n
+    keep = (DUMP_LIMIT_BYTES - 1024 * len(arrays)) // row_bytes     # 1 KiB per file covers the .npy header
+    if keep < n:
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def algorithmic_flops_per_env_step(nj, nc_sum, sweep_feet, frame_skip=4):
@@ -290,8 +310,10 @@ def run_reference(args):
         v.step(acts[i % 8])
     t0 = time.perf_counter()
     for i in range(args.steps):
-        v.step(acts[i % 8])
+        obs, rew, done = v.step(acts[i % 8])
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"obs": obs, "reward": rew, "done": done})
     val = n * args.steps / dt
     sample = (f"{n} envs per step (the GPU arm's batch) on {nthreads} host threads; fp64 CPU restatement (oracle/), "
               f"PyBullet itself is not installable in this image; " + CPU_RESET_NOTE)
@@ -627,7 +649,7 @@ def run_ours(args):
     for i in range(args.steps):
         flush.fill_(float(i))
         evs[i][0].record()
-        sim.step(acts[i % nact])
+        out = sim.step(acts[i % nact])
         evs[i][1].record()
     barrier()
     t_wall = time.perf_counter() - t_wall0
@@ -635,6 +657,8 @@ def run_ours(args):
     clocks = sampler.stop()
     step_ms = np.array([a.elapsed_time(b) for a, b in evs])
     total_ms = float(step_ms.sum())
+    if args.dump_outputs and rank == 0:       # the step's buffers are overwritten by the steps below
+        dump_outputs(args.dump_outputs, {k: t.cpu().numpy() for k, t in zip(("obs", "reward", "done"), out)})
     for i in range(16):
         _, _, d, _ = env.step(acts[i % nact])
         sample_work(d)
@@ -802,7 +826,11 @@ def main():
     ap.add_argument("--no-ppo-train", action="store_true")
     ap.add_argument("--no-saturated", action="store_true")
     ap.add_argument("--saturated-envs", type=int, default=65536)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write obs/reward/done of the last timed step as DIR/<name>.npy (float32, at most 64 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -176,13 +176,11 @@ def test_shipped_configs_keep_the_reference_keys(name, robot, task, control, H):
     from solorl_b200.abi import dims, params_from_config, _TASK_NAMES, _CONTROL_NAMES
     from solorl_b200.model import SoloModel
     cfg = yaml.safe_load(open(os.path.join(ROOT, "configs", name + ".yaml")))
-    ref_path = os.path.join("/root/reference/configs", name + ".yaml")
-    if os.path.exists(ref_path):
-        ref = yaml.safe_load(open(ref_path))
-        assert set(cfg) == set(ref)
-        for k in ref:
-            if k != "model_urdf":
-                assert cfg[k] == ref[k], k
+    ref = json.load(open(os.path.join(GOLDEN, "reference_configs.json")))[name]    # the reference's configs/<name>.yaml
+    assert set(cfg) == set(ref)
+    for k in ref:
+        if k != "model_urdf":
+            assert cfg[k] == ref[k], k
     m = SoloModel.resolve(cfg["model_urdf"])
     p = params_from_config(cfg, m)
     assert m.name == robot and p.task == _TASK_NAMES[task] and p.control == _CONTROL_NAMES[control]

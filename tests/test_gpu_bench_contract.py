@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 from tests.helpers import ROOT
@@ -50,6 +51,23 @@ def test_bench_line_has_every_contract_key():
     ps = d["ppo_stand"]
     assert ps["seconds_to_target"] is not None and ps["seconds_to_target"] < 300 and ps["final_return"] >= ps["target_return"]
     assert d["body_contacts"]["value"] > 0 and d["gae"]["frac"] > 0.1 and d["reset_mode_simulate"]["value"] > 0
+
+
+def test_dump_outputs_of_the_last_timed_step(tmp_path):
+    """--dump-outputs writes obs / reward / done of the last of exactly --steps timed steps; the same arguments give
+    the same inputs, hence the same outputs, run after run."""
+    quick = ("--warmup", "3", "--no-cpu-baseline", "--no-policy-rollout", "--no-ppo-train", "--no-saturated")
+    dumps = {}
+    for tag, steps in (("a", 7), ("b", 7), ("c", 8)):
+        d = _run("--steps", str(steps), *quick, "--dump-outputs", str(tmp_path / tag))
+        assert d["steps"] == steps and d["gpu_launches"] == steps
+        dumps[tag] = {k: np.load(tmp_path / tag / (k + ".npy")) for k in ("obs", "reward", "done")}
+    a = dumps["a"]
+    assert a["obs"].shape == (4096, 76) and a["reward"].shape == (4096,) and a["done"].shape == (4096,)
+    assert all(x.dtype == np.float32 for x in a.values()) and np.isfinite(a["obs"]).all()
+    for k in a:
+        assert np.array_equal(a[k], dumps["b"][k]), k
+    assert not np.array_equal(a["obs"], dumps["c"]["obs"])
 
 
 def test_reference_arm_line():

@@ -1,4 +1,5 @@
 """Model table known answers (SURVEY Appendix A) and the URDF parser."""
+import json
 import os
 
 import numpy as np
@@ -6,8 +7,7 @@ import pytest
 
 from solorl_b200.abi import model_table
 from solorl_b200.model import JOINT_FIXED, JOINT_REVOLUTE, SoloModel
-
-REF = "/root/reference/solo_description/robots"
+from tests.helpers import GOLDEN
 
 
 def test_solo8_table():
@@ -86,11 +86,12 @@ def test_resolve_reference_config_paths():
         SoloModel.resolve("/nowhere/other.urdf")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
 @pytest.mark.parametrize("urdf,name", [("solo.urdf", "solo8"), ("solo12.urdf", "solo12")])
 def test_builtin_equals_reference_urdf(urdf, name):
-    a = SoloModel.from_urdf(os.path.join(REF, urdf))
+    # the fields SoloModel.from_urdf reads off the reference's solo_description/robots/<urdf>, stored as golden data
+    with open(os.path.join(GOLDEN, "reference_urdf_models.json")) as f:
+        a = json.load(f)[urdf]
     b = SoloModel.builtin(name)
-    assert a.joint_names == b.joint_names and a.parent == b.parent and a.jtype == b.jtype
+    assert a["joint_names"] == b.joint_names and a["parent"] == b.parent and a["jtype"] == b.jtype
     for f in ("axis", "origin", "mass", "com", "inertia", "base_inertia"):
-        assert np.array_equal(getattr(a, f), getattr(b, f)), f
+        assert np.array_equal(np.array(a[f], dtype=np.float64), getattr(b, f)), f
