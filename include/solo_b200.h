@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define SOLO_ABI_VERSION 1
+#define SOLO_ABI_VERSION 2
 
 #define SOLO_MAX_LINKS 20
 #define SOLO_MAX_FEET 4
@@ -157,6 +157,21 @@ typedef struct SoloSimParams {
   double knee_radius;             /* 0.015: the lower-leg mesh reaches 0.0135 m above the KFE axis (SURVEY App. A) */
   double base_half_x, base_half_y;/* 0.2241 x 0.1095 (Solo12), 0.212 x 0.1046 (Solo8) */
   double base_z_lo, base_z_hi;    /* -0.025, 0.028: bottom / top of the base box relative to the base origin */
+  /* Randomised dynamics (domain randomisation for sim-to-real).  With randomize = 1 every reset (full, masked,
+   * or the auto-reset inside solo_step) draws three values per env, each uniform in [lo, hi] from the env's own
+   * RNG stream, fixed for the episode:
+   *   friction        the combined lateral friction of the env's contact rows (replaces `friction`);
+   *   base_mass_scale base mass and base inertia tensor times this (the legs keep theirs);
+   *   motor_strength  the torque of every action mode times this (max_torque; kp, kd and the clamp under PD / VPD).
+   * They act in the control steps of solo_step / solo_step_host, solo_substep, solo_forward_dynamics and
+   * solo_action_to_torque.  The settle steps of a reset run with the nominal values (so cached resets stay
+   * exact); solo_actuator_step (gait envs) does not use them.  Not available in the wide build.
+   * randomize = 0 (default): the ranges are not read.  With randomize = 1 all six bounds must be set
+   * (0 <= friction_lo <= friction_hi, 0 < lo <= hi for the scales); solo_default_params leaves them 0. */
+  int32_t randomize;
+  double friction_lo, friction_hi;
+  double base_mass_scale_lo, base_mass_scale_hi;
+  double motor_strength_lo, motor_strength_hi;
 } SoloSimParams;
 
 /* Per-env episode record, valid for envs whose `done` was 1 at the last step
@@ -252,15 +267,21 @@ int solo_forward_dynamics(SoloHandle* h, const float* d_state, const float* d_ta
 int solo_substep(SoloHandle* h, const float* d_tau, void* stream);
 
 /* Action -> joint torque exactly as solo.py:224-259 + controllers/PD.py:3-10 on the
- * handle's current state. d_tau [N, nj]. */
+ * handle's current state (times the env's motor strength on a randomised handle). d_tau [N, nj]. */
 int solo_action_to_torque(SoloHandle* h, const float* d_actions, float* d_tau, void* stream);
+
+/* The dynamics each env runs its episode with, d_out float[N, 3] = (friction, base_mass_scale, motor_strength):
+ * the values the last reset drew on a randomised handle (privileged critic inputs, logging), the nominal
+ * (friction, 1, 1) otherwise and before the first reset. */
+int solo_get_env_params(SoloHandle* h, float* d_out, void* stream);
 
 /* Gait envs (SURVEY §8f n2): n_ticks simulator ticks under the joint-level PD + feed-forward actuator
  * that the external PyBulletSimulator exposes to baseControlEnv.py:256-270
  * (SetDesiredJointPDgains / Position / Velocity / Torque + SendCommand):
  *   tau = clip(P (q_des - q) + D (v_des - v) + tau_ff, +-max_torque), recomputed before every tick,
  * then one Bullet-equivalent step at params.dt (create the handle with dt = 0.002, the gait envs' tick).
- * d_cmd float[N, 5, nj] = q_des, v_des, P, D, tau_ff.  State is read back with solo_get_state. */
+ * d_cmd float[N, 5, nj] = q_des, v_des, P, D, tau_ff.  State is read back with solo_get_state.
+ * Runs with the nominal dynamics: SoloSimParams.randomize does not apply to the gait envs. */
 int solo_actuator_step(SoloHandle* h, const float* d_cmd, int32_t n_ticks, void* stream);
 
 /* Gait envs: external force on the base for the following solo_actuator_step calls, d_force float[N, 3] in base
@@ -301,8 +322,8 @@ int solo_gae(const float* d_rewards, const float* d_values, const float* d_masks
 int64_t solo_launch_count(const SoloHandle* h);
 
 /* Which build of the step kernel this handle launches ("latency", "throughput", "wide", or "body" when
- * SoloSimParams.body_contacts is set): chosen at create time from the batch size, SOLO_STEP_VARIANT overrides
- * (bench / profile evidence). */
+ * SoloSimParams.body_contacts is set; "+rand" appended on a randomised handle): chosen at create time from the
+ * batch size, SOLO_STEP_VARIANT overrides (bench / profile evidence). */
 const char* solo_step_variant(const SoloHandle* h);
 
 #ifdef __cplusplus

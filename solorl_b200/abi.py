@@ -10,7 +10,7 @@ import numpy as np
 
 from .model import SoloModel
 
-ABI_VERSION = 1
+ABI_VERSION = 2
 MAX_LINKS = 20
 MAX_FEET = 4
 
@@ -94,6 +94,13 @@ class SoloSimParams(C.Structure):
         ("base_half_y", C.c_double),
         ("base_z_lo", C.c_double),
         ("base_z_hi", C.c_double),
+        ("randomize", C.c_int32),
+        ("friction_lo", C.c_double),
+        ("friction_hi", C.c_double),
+        ("base_mass_scale_lo", C.c_double),
+        ("base_mass_scale_hi", C.c_double),
+        ("motor_strength_lo", C.c_double),
+        ("motor_strength_hi", C.c_double),
     ]
 
 
@@ -205,7 +212,45 @@ def default_params() -> SoloSimParams:
     p.knee_radius = 0.015
     p.base_half_x, p.base_half_y = 0.2241, 0.1095
     p.base_z_lo, p.base_z_hi = -0.025, 0.028
+    # randomised dynamics off; the ranges are only read with randomize = 1 (params_from_config sets them)
+    p.randomize = 0
+    p.friction_lo = p.friction_hi = 0.0
+    p.base_mass_scale_lo = p.base_mass_scale_hi = 0.0
+    p.motor_strength_lo = p.motor_strength_hi = 0.0
     return p
+
+
+# config key -> (SoloSimParams range fields, nominal value (None: the params' friction), lower bound is exclusive)
+_RANDOMIZE_KEYS = {
+    "randomize_friction": ("friction_lo", "friction_hi", None, False),
+    "randomize_base_mass": ("base_mass_scale_lo", "base_mass_scale_hi", 1.0, True),
+    "randomize_motor_strength": ("motor_strength_lo", "motor_strength_hi", 1.0, True),
+}
+
+
+def _randomize_from_config(config: dict, p: SoloSimParams) -> None:
+    """Per-env randomised dynamics: ``randomize_friction``, ``randomize_base_mass`` and
+    ``randomize_motor_strength``, each ``[lo, hi]``.  Any of them present sets ``randomize``; a missing one
+    keeps its value at the nominal (friction, 1, 1).  Malformed ranges raise ``ValueError``."""
+    if not any(k in config for k in _RANDOMIZE_KEYS):
+        return
+    p.randomize = 1
+    for key, (f_lo, f_hi, nominal, positive) in _RANDOMIZE_KEYS.items():
+        if key not in config:
+            v = p.friction if nominal is None else nominal
+            setattr(p, f_lo, v)
+            setattr(p, f_hi, v)
+            continue
+        r = config[key]
+        try:
+            lo, hi = (float(x) for x in r)
+        except (TypeError, ValueError):
+            raise ValueError(f"{key} must be a list [lo, hi] of two numbers, got {r!r}") from None
+        if not (np.isfinite(lo) and np.isfinite(hi)) or lo > hi or lo < 0 or (positive and lo == 0):
+            bound = "0 < lo <= hi" if positive else "0 <= lo <= hi"
+            raise ValueError(f"{key}: [{lo}, {hi}] must satisfy {bound}")
+        setattr(p, f_lo, lo)
+        setattr(p, f_hi, hi)
 
 
 def params_from_config(config: dict, model: Optional[SoloModel] = None) -> SoloSimParams:
@@ -215,7 +260,9 @@ def params_from_config(config: dict, model: Optional[SoloModel] = None) -> SoloS
     ``episode_length`` (required), ``frame_skip`` 4, ``control`` 'torque', ``task``
     'stand', ``gains`` None, ``num_history_stack`` 0, ``flat_ground`` True,
     ``use_treadmill`` False.  Extra keys (all default to the reference-faithful value):
-    ``torque_hold``, ``solver_iters``, ``solver_residual_threshold``, ``contact_erp``, ``reset_mode``.
+    ``torque_hold``, ``solver_iters``, ``solver_residual_threshold``, ``contact_erp``, ``reset_mode``;
+    ``randomize_friction``, ``randomize_base_mass``, ``randomize_motor_strength`` (per-env randomised
+    dynamics, see ``_randomize_from_config``).
     """
     p = default_params()
     p.episode_length = int(config["episode_length"])           # baseEnv.py:164 (required)
@@ -256,6 +303,7 @@ def params_from_config(config: dict, model: Optional[SoloModel] = None) -> SoloS
             setattr(p, k, float(config[k]))
     rm = config.get("reset_mode", "cached")
     p.reset_mode = {"cached": RESET_CACHED, "simulate": RESET_SIMULATE}[rm]
+    _randomize_from_config(config, p)
     return p
 
 

@@ -284,7 +284,8 @@ __device__ __forceinline__ void body_apply_me(const BodyRowR& r, float d, bool m
 }
 template <bool CONE>
 __device__ __forceinline__ int body_pgs_lanes(float* rows, unsigned lmask, unsigned pmask, const SimConst& sc,
-                                              unsigned gmask, unsigned gbase, int me, float* dv0, float* s_me) {
+                                              unsigned gmask, unsigned gbase, int me, float* dv0, float* s_me,
+                                              const EnvDyn* dyn = nullptr) {
 #pragma unroll
   for (int i = 0; i < 6; i++) dv0[i] = 0.f;
   s_me[0] = s_me[1] = s_me[2] = 0.f;
@@ -345,7 +346,7 @@ __device__ __forceinline__ int body_pgs_lanes(float* rows, unsigned lmask, unsig
       float* rn = rows + body_slot(p, 0) * kBodyRowW;
       float* ra = rn + kBodyRowW;
       float* rb = ra + kBodyRowW;
-      const float lim = sc.mu * rn[kBrLam];
+      const float lim = env_mu(sc, dyn) * rn[kBrLam];
       BodyRowR A, B;
       body_row_load(ra, A);
       body_row_load(rb, B);

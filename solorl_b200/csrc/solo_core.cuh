@@ -83,6 +83,14 @@ struct SimConst {
   float knee_r, base_hx, base_hy, base_zlo, base_zhi;
 };
 
+/* Dynamics of one env of a randomised handle (SoloSimParams.randomize): contact friction, base mass / inertia
+ * scale, motor strength.  Wherever a `const EnvDyn*` is taken, nullptr means the nominal values of SimConst /
+ * ModelConst, and the code is then exactly that of a handle without randomisation. */
+struct EnvDyn {
+  float mu, sm, st;
+};
+SOLO_HD float env_mu(const SimConst& sc, const EnvDyn* dyn) { return dyn != nullptr ? dyn->mu : sc.mu; }
+
 /* ------------------------------------------------------------------ small helpers */
 SOLO_HD float dot3(const float* a, const float* b) { return a[0] * b[0] + a[1] * b[1] + a[2] * b[2]; }
 SOLO_HD void cross3(const float* a, const float* b, float* o) {
@@ -554,14 +562,27 @@ SOLO_HD void leg_inward(const LegConst& lc, const SimConst& sc, const BaseWork& 
   leg_recursion<NJL>(lc, ln, tau, pk, com, Ic, IAleg, pAleg);
 }
 
-/* Base rigid body: add to the summed leg inertias / bias, factor, solve a0 = -IA0^-1 pA0. */
-SOLO_HD void base_solve(const ModelConst& mc, const SimConst& sc, BaseWork& bw, Sym6& IA0,
-                        float* pA0, float* a0) {
+/* The base body's inertia added to IA0, its angular momentum (base axes) nb and linear momentum l. */
+SOLO_HD void base_rigid(float m, const float* I, const BaseWork& bw, Sym6& IA0, float* nb, float* l) {
   const float zero3[3] = {0.f, 0.f, 0.f};
-  sym6_add_rigid(IA0, mc.base_m, zero3, mc.base_I);
+  sym6_add_rigid(IA0, m, zero3, I);
+  sym3_mulv(I, bw.wb, nb);
+  l[0] = m * bw.vb[0]; l[1] = m * bw.vb[1]; l[2] = m * bw.vb[2];
+}
+
+/* Base rigid body: add to the summed leg inertias / bias, factor, solve a0 = -IA0^-1 pA0.
+ * dyn: base mass and inertia scaled by dyn->sm (randomised dynamics). */
+SOLO_HD void base_solve(const ModelConst& mc, const SimConst& sc, BaseWork& bw, Sym6& IA0,
+                        float* pA0, float* a0, const EnvDyn* dyn = nullptr) {
   float nb[3], l[3];
-  sym3_mulv(mc.base_I, bw.wb, nb);
-  l[0] = mc.base_m * bw.vb[0]; l[1] = mc.base_m * bw.vb[1]; l[2] = mc.base_m * bw.vb[2];
+  if (dyn == nullptr) {
+    base_rigid(mc.base_m, mc.base_I, bw, IA0, nb, l);
+  } else {
+    float I[6];
+#pragma unroll
+    for (int i = 0; i < 6; i++) I[i] = mc.base_I[i] * dyn->sm;
+    base_rigid(mc.base_m * dyn->sm, I, bw, IA0, nb, l);
+  }
   float sa = sc.kang + sc.kang * solo_sqrt_approx(dot3(bw.wb, bw.wb));
   float sl = sc.klin + sc.klin * solo_sqrt_approx(dot3(bw.vb, bw.vb));
   float pb[6];

@@ -117,6 +117,30 @@ SOLO_HD void book_clear_episode(EnvBook& bk) { /* baseEnv.py:72-77 */
   for (int i = 0; i < 5; i++) bk.dr[i] = 0.f;
 }
 
+/* Ranges of the randomised dynamics (SoloSimParams.friction_lo .. motor_strength_hi, narrowed to float). */
+struct EnvRanges {
+  float mu_lo, mu_hi, sm_lo, sm_hi, st_lo, st_hi;
+};
+
+/* Philox draw index of the dynamics draw: the per-episode draws (settle count and goal at the reset, new goals while
+ * stepping) count up from 0 and never reach it, so they stay what they are without randomisation. */
+constexpr uint32_t kDynDraw = 0x80000000u;
+
+/* The dynamics of env `gid` for episode `episode`: each value uniform in its range.  fmaf keeps the device and a
+ * host replay bit-identical; fminf keeps a rounded-up product inside the range. */
+SOLO_HD float dyn_uniform(float lo, float hi, uint32_t w) { return fminf(fmaf(hi - lo, u01(w), lo), hi); }
+SOLO_HD EnvDyn sample_env_dyn(const EnvRanges& r, uint32_t seed_lo, uint32_t seed_hi, long long gid,
+                              uint32_t episode) {
+  uint32_t w[4] = {(uint32_t)((unsigned long long)gid & 0xffffffffull), (uint32_t)((unsigned long long)gid >> 32),
+                   episode, kDynDraw};
+  philox4x32_10(w, seed_lo, seed_hi);
+  EnvDyn p;
+  p.mu = dyn_uniform(r.mu_lo, r.mu_hi, w[0]);
+  p.sm = dyn_uniform(r.sm_lo, r.sm_hi, w[1]);
+  p.st = dyn_uniform(r.st_lo, r.st_hi, w[2]);
+  return p;
+}
+
 /* robot_specific_reset (solo.py:291-296): base -> (0,0,initial_z), identity, zero velocity */
 SOLO_HD void reset_pose(const SimConst& sc, BaseState& st) {
   st.p[0] = 0.f; st.p[1] = 0.f; st.p[2] = sc.initial_z;

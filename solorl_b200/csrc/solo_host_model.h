@@ -14,6 +14,7 @@
 
 #include "../../include/solo_b200.h"
 #include "solo_core.cuh"
+#include "solo_env.cuh"
 
 namespace solo {
 
@@ -125,6 +126,25 @@ inline int build_sim_const(const SoloSimParams& p, SimConst& sc, std::string& er
   }
   sc.knee_r = (float)p.knee_radius; sc.base_hx = (float)p.base_half_x; sc.base_hy = (float)p.base_half_y;
   sc.base_zlo = (float)p.base_z_lo; sc.base_zhi = (float)p.base_z_hi;
+  return SOLO_OK;
+}
+
+/* Ranges of the randomised dynamics, checked when SoloSimParams.randomize is set (and left 0 otherwise). */
+inline int build_env_ranges(const SoloSimParams& p, EnvRanges& r, std::string& err) {
+  memset(&r, 0, sizeof(r));
+  if (!p.randomize) return SOLO_OK;
+  if (!(p.friction_lo >= 0 && p.friction_lo <= p.friction_hi)) {
+    err = "randomize: friction range must satisfy 0 <= friction_lo <= friction_hi"; return SOLO_E_ARG;
+  }
+  if (!(p.base_mass_scale_lo > 0 && p.base_mass_scale_lo <= p.base_mass_scale_hi)) {
+    err = "randomize: base mass scale range must satisfy 0 < lo <= hi"; return SOLO_E_ARG;
+  }
+  if (!(p.motor_strength_lo > 0 && p.motor_strength_lo <= p.motor_strength_hi)) {
+    err = "randomize: motor strength range must satisfy 0 < lo <= hi"; return SOLO_E_ARG;
+  }
+  r.mu_lo = (float)p.friction_lo; r.mu_hi = (float)p.friction_hi;
+  r.sm_lo = (float)p.base_mass_scale_lo; r.sm_hi = (float)p.base_mass_scale_hi;
+  r.st_lo = (float)p.motor_strength_lo; r.st_hi = (float)p.motor_strength_hi;
   return SOLO_OK;
 }
 

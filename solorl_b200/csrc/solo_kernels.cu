@@ -83,6 +83,14 @@ struct StepArgs {
   int force_settle;   /* >=0: cache generation, env i settles settle_min + i steps, goal far away */
 };
 
+/* Randomised dynamics of a handle: per-env (mu, base mass scale, motor strength, 0) and the ranges a reset draws
+ * them from; envp == nullptr: randomisation off.  A kernel parameter of its own, after StepArgs, so that the
+ * kernels without randomisation keep their parameter layout. */
+struct DynArgs {
+  float4* envp;
+  EnvRanges ranges;
+};
+
 struct ResetArgs {
   DevArrays d;
   SimConst sc;
@@ -92,6 +100,7 @@ struct ResetArgs {
   uint32_t seed_lo, seed_hi;
   long long env_id_offset;
   int reset_simulate, force_settle;
+  DynArgs dyn;
 };
 
 /* Observation rows of the eight envs of a warp are assembled in shared memory and leave the SM as
@@ -251,10 +260,15 @@ template <int NJL>
 __device__ __forceinline__ void begin_reset(const DevArrays& d, const SimConst& sc, int D0, int e, int leg,
                                             long long gid, uint32_t seed_lo, uint32_t seed_hi, float goal_radius,
                                             int reset_simulate, int force_settle, BaseState& st, Lane<NJL>& ln,
-                                            float& cforce, float* goal, float& potential, EnvBook& bk) {
+                                            float& cforce, float* goal, float& potential, EnvBook& bk,
+                                            const DynArgs* dyn = nullptr) {
   bk.episode += 1; bk.draw = 0;
   uint32_t w[4];
   env_rng(seed_lo, seed_hi, gid, bk, w);
+  if (dyn != nullptr && dyn->envp != nullptr && leg == 0) {    /* the new episode's dynamics */
+    const EnvDyn p = sample_env_dyn(dyn->ranges, seed_lo, seed_hi, gid, bk.episode);
+    dyn->envp[e] = make_float4(p.mu, p.sm, p.st, 0.f);
+  }
   if (sc.task == 2) sample_goal(w, goal_radius, goal);          /* solo.py:173-174 */
   int k = sc.settle_min + (sc.settle_span > 0 ? (int)(w[0] % (uint32_t)sc.settle_span) : 0); /* baseEnv.py:79 */
   if (force_settle >= 0) { k = sc.settle_min + (e % (sc.settle_span > 0 ? sc.settle_span : 1)); goal[0] = 1.0e3f; goal[1] = 1.0e3f; }
@@ -299,7 +313,7 @@ __device__ __forceinline__ void begin_reset(const DevArrays& d, const SimConst& 
  * stopping there.  CONE selects Bullet's implicit-cone friction rows or the pyramid ones. */
 template <bool CONE>
 __device__ __forceinline__ void pgs_sweeps(PgsLane& pl, const SimConst& sc, int leg, unsigned gbase, unsigned amask,
-                                           int nc, float* lam3, int& sweep_feet) {
+                                           int nc, float* lam3, int& sweep_feet, const EnvDyn* dyn) {
   const unsigned kFull = 0xffffffffu;
   bool conv = (amask == 0);          /* env-uniform: the sweep loop of this env has ended */
   lam3[0] = lam3[1] = lam3[2] = 0.f;
@@ -320,7 +334,7 @@ __device__ __forceinline__ void pgs_sweeps(PgsLane& pl, const SimConst& sc, int 
     for (int f = 0; f < 4; f++) {
       if (CONE) {
         float nA, nB, dA, dB, rv;
-        pgs_cone_candidate(pl, sc.mu, nA, nB, dA, dB, rv);
+        pgs_cone_candidate(pl, env_mu(sc, dyn), nA, nB, dA, dB, rv);
         const float dAb = __shfl_sync(kFull, dA, gbase + f);
         const float dBb = __shfl_sync(kFull, dB, gbase + f);
         if (leg == f) { pl.lam[1] = nA; pl.lam[2] = nB; res_own = fmaxf(res_own, fabsf(rv)); }
@@ -330,7 +344,7 @@ __device__ __forceinline__ void pgs_sweeps(PgsLane& pl, const SimConst& sc, int 
 #pragma unroll
         for (int q = 0; q < 2; q++) {
           float nv, d, rv;
-          pgs_pyramid_candidate(pl, sc.mu, q, nv, d, rv);
+          pgs_pyramid_candidate(pl, env_mu(sc, dyn), q, nv, d, rv);
           const float db = __shfl_sync(kFull, d, gbase + f);
           if (leg == f) { pl.lam[1 + q] = nv; res_own = fmaxf(res_own, fabsf(rv)); }
           pgs_apply(pl, row_of(f, 1 + q), db);
@@ -351,7 +365,8 @@ __device__ __forceinline__ void pgs_sweeps(PgsLane& pl, const SimConst& sc, int 
  * every sweep like Bullet's non-contact rows (under random actions 11 % of env steps hold a limit row). */
 template <bool CONE>
 __device__ __forceinline__ void pgs_sweeps4(PgsLane4& pl, const SimConst& sc, int leg, unsigned gbase, unsigned amask,
-                                            unsigned lmask, unsigned lwarp, int nc, float* lam4, int& sweep_feet) {
+                                            unsigned lmask, unsigned lwarp, int nc, float* lam4, int& sweep_feet,
+                                            const EnvDyn* dyn) {
   const unsigned kFull = 0xffffffffu;
   bool conv = (amask == 0) && (lmask == 0);
   lam4[0] = lam4[1] = lam4[2] = lam4[3] = 0.f;
@@ -390,7 +405,7 @@ __device__ __forceinline__ void pgs_sweeps4(PgsLane4& pl, const SimConst& sc, in
     for (int f = 0; f < 4; f++) {
       if (CONE) {
         float nA, nB, dA, dB, rv;
-        pgs_cone_candidate(pl, sc.mu, nA, nB, dA, dB, rv);
+        pgs_cone_candidate(pl, env_mu(sc, dyn), nA, nB, dA, dB, rv);
         const float dAb = __shfl_sync(kFull, dA, gbase + f);
         const float dBb = __shfl_sync(kFull, dB, gbase + f);
         if (leg == f) { pl.lam[1] = nA; pl.lam[2] = nB; res_own = fmaxf(res_own, fabsf(rv)); }
@@ -400,7 +415,7 @@ __device__ __forceinline__ void pgs_sweeps4(PgsLane4& pl, const SimConst& sc, in
 #pragma unroll
         for (int q = 0; q < 2; q++) {
           float nv, d, rv;
-          pgs_pyramid_candidate(pl, sc.mu, q, nv, d, rv);
+          pgs_pyramid_candidate(pl, env_mu(sc, dyn), q, nv, d, rv);
           const float db = __shfl_sync(kFull, d, gbase + f);
           if (leg == f) { pl.lam[1 + q] = nv; res_own = fmaxf(res_own, fabsf(rv)); }
           pgs_apply(pl, row_of(f, 1 + q), db);
@@ -433,7 +448,7 @@ template <int NJL, bool LIMITS, bool BODY>
 __device__ __forceinline__ void contact_solve(const SimConst& sc, int leg, BaseState& st, const BaseWork& bw,
                                               Lane<NJL>& ln, bool lim_env, int kL, float dirL, float penL,
                                               float& cforce, int& nc_sum, int& sweep_feet, int g_trace_sub = 0,
-                                              float* body_rows = nullptr) {
+                                              float* body_rows = nullptr, const EnvDyn* dyn = nullptr) {
   const unsigned kFull = 0xffffffffu;
   const unsigned lane = threadIdx.x & 31u;
   const unsigned gbase = lane & ~3u;
@@ -492,8 +507,8 @@ __device__ __forceinline__ void contact_solve(const SimConst& sc, int leg, BaseS
     nc_sum += nc;
     float lam4[4];
     NSTAMP(3);
-    if (sc.cone) pgs_sweeps4<true>(pl, sc, leg, gbase, amask, lmask, lwarp, nc, lam4, sweep_feet);
-    else pgs_sweeps4<false>(pl, sc, leg, gbase, amask, lmask, lwarp, nc, lam4, sweep_feet);
+    if (sc.cone) pgs_sweeps4<true>(pl, sc, leg, gbase, amask, lmask, lwarp, nc, lam4, sweep_feet, dyn);
+    else pgs_sweeps4<false>(pl, sc, leg, gbase, amask, lmask, lwarp, nc, lam4, sweep_feet, dyn);
     NSTAMP(4);
     lam3[0] = lam4[0]; lam3[1] = lam4[1]; lam3[2] = lam4[2];
     float part[6], dv0[6];
@@ -523,8 +538,8 @@ __device__ __forceinline__ void contact_solve(const SimConst& sc, int leg, BaseS
     }
     const int nc = __popc(amask);
     nc_sum += nc;
-    if (sc.cone) pgs_sweeps<true>(pl, sc, leg, gbase, amask, nc, lam3, sweep_feet);
-    else pgs_sweeps<false>(pl, sc, leg, gbase, amask, nc, lam3, sweep_feet);
+    if (sc.cone) pgs_sweeps<true>(pl, sc, leg, gbase, amask, nc, lam3, sweep_feet, dyn);
+    else pgs_sweeps<false>(pl, sc, leg, gbase, amask, nc, lam3, sweep_feet, dyn);
     float part[6], dv0[6];
     impulse_base_part<NJL>(ln, lam3, part);
 #pragma unroll
@@ -546,8 +561,8 @@ __device__ __forceinline__ void contact_solve(const SimConst& sc, int leg, BaseS
       body_lane_fill<NJL>(sc, st, bw, ln, LIMITS ? &lr : nullptr, leg, foot_on != 0, bg, body_rows);
       __syncwarp(gmask);
       float dv0[6], us[3];
-      const int sweeps = sc.cone ? body_pgs_lanes<true>(body_rows, lm_all, pmask, sc, gmask, gbase, leg, dv0, us)
-                                 : body_pgs_lanes<false>(body_rows, lm_all, pmask, sc, gmask, gbase, leg, dv0, us);
+      const int sweeps = sc.cone ? body_pgs_lanes<true>(body_rows, lm_all, pmask, sc, gmask, gbase, leg, dv0, us, dyn)
+                                 : body_pgs_lanes<false>(body_rows, lm_all, pmask, sc, gmask, gbase, leg, dv0, us, dyn);
       body_apply_leg<NJL>(ln, sc, us, dv0);
       float dw[3], dvl[3];
       mat3_mulv(bw.R, dv0, dw);
@@ -575,7 +590,8 @@ template <int NJL, bool LIMITS, bool BODY = false>
 __device__ __forceinline__ void group_substep(const LegConst& lc, const ModelConst& mc, const SimConst& sc,
                                               int leg, BaseState& st, Lane<NJL>& ln, const float* tau, float& cforce,
                                               int& nc_sum, int& sweep_feet, int g_trace_sub = 0,
-                                              const float* fext = nullptr, float* body_rows = nullptr) {
+                                              const float* fext = nullptr, float* body_rows = nullptr,
+                                              const EnvDyn* dyn = nullptr) {
   NSTAMP(0);
   BaseWork bw;
   base_prepare(st, bw);
@@ -589,7 +605,7 @@ __device__ __forceinline__ void group_substep(const LegConst& lc, const ModelCon
 #pragma unroll
     for (int i = 0; i < 3; i++) pA[3 + i] -= fext[i];
   }
-  base_solve(mc, sc, bw, IA, pA, a0);
+  base_solve(mc, sc, bw, IA, pA, a0, dyn);
   {
     float qdd[NJL], aw[3], al[3];
     leg_outward<NJL>(ln, a0, qdd);
@@ -606,7 +622,7 @@ __device__ __forceinline__ void group_substep(const LegConst& lc, const ModelCon
   float dirL, penL;
   const bool lim_any = LIMITS && limit_select<NJL>(sc, ln, kL, dirL, penL);
   contact_solve<NJL, LIMITS, BODY>(sc, leg, st, bw, ln, lim_any, kL, dirL, penL, cforce, nc_sum, sweep_feet, g_trace_sub,
-                                   body_rows);
+                                   body_rows, dyn);
   NSTAMP(5);
 }
 
@@ -619,6 +635,7 @@ struct EnvLane {
   float cforce;
   EnvBook bk;
   float tau[NJL], act[NJL];
+  EnvDyn dyn;          /* RAND builds only */
   int e, el, leg, tid;
   long long gid;
   bool valid, active;
@@ -627,8 +644,9 @@ typedef float StageTile[8][kStageD];
 
 /* Step prologue of one lane: state load, apply_action (solo.py:224-259), history push (solo.py:262).
  * wslot = index of this lane's warp among the env warps of the grid (eight envs per warp). */
-template <int NJL>
-__device__ __forceinline__ void step_load(const StepArgs& args, int wslot, int tid, StageTile& stage, EnvLane<NJL>& L) {
+template <int NJL, bool RAND = false>
+__device__ __forceinline__ void step_load(const StepArgs& args, int wslot, int tid, StageTile& stage, EnvLane<NJL>& L,
+                                          const DynArgs* dyn = nullptr) {
   const SimConst& sc = args.sc;
   const DevArrays& d = args.d;
   L.tid = tid;
@@ -647,6 +665,11 @@ __device__ __forceinline__ void step_load(const StepArgs& args, int wslot, int t
   L.cforce = d.cforce[e * 4 + leg];
   L.bk = d.book[e];
   L.active = L.valid && (args.mode != MODE_SETTLE || L.bk.settle_left > 0);
+  if (RAND) {
+    /* the settle steps of a reset run with the nominal dynamics, so that a cached reset stays exact */
+    if (args.mode == MODE_SETTLE) { L.dyn.mu = sc.mu; L.dyn.sm = 1.f; L.dyn.st = 1.f; }
+    else { const float4 p = dyn->envp[e]; L.dyn.mu = p.x; L.dyn.sm = p.y; L.dyn.st = p.z; }
+  }
 #pragma unroll
   for (int k = 0; k < NJL; k++) { L.tau[k] = 0.f; L.act[k] = 0.f; }
   if (args.mode == MODE_STEP) {                     /* apply_action (solo.py:224-259) */
@@ -669,6 +692,7 @@ __device__ __forceinline__ void step_load(const StepArgs& args, int wslot, int t
     for (int k = 0; k < NJL; k++) {
       L.act[k] = a[leg * NJL + k];
       L.tau[k] = action_to_torque(sc, L.act[k], L.ln.q[k], L.ln.qd[k], kp, kd);
+      if (RAND) L.tau[k] *= L.dyn.st;
     }
     __syncwarp();                                   /* the stage is reused for the observation rows */
   } else if (args.mode == MODE_SUBSTEP) {
@@ -685,8 +709,9 @@ __device__ __forceinline__ void step_load(const StepArgs& args, int wslot, int t
 
 /* Step epilogue of one lane: pointgoal bookkeeping (solo.py:267-272), observation, reward / termination
  * (baseEnv.py:47-68), episode record, worker auto-reset (agents/ppo/envs.py:38-40), state store. */
-template <int NJL>
-__device__ __forceinline__ void step_finish(const StepArgs& args, int wslot, StageTile& stage, EnvLane<NJL>& L) {
+template <int NJL, bool RAND = false>
+__device__ __forceinline__ void step_finish(const StepArgs& args, int wslot, StageTile& stage, EnvLane<NJL>& L,
+                                            const DynArgs* dyn = nullptr) {
   const SimConst& sc = args.sc;
   const DevArrays& d = args.d;
   const int e = L.e, leg = L.leg, el = L.el, tid = L.tid, D0 = args.D0;
@@ -745,7 +770,7 @@ __device__ __forceinline__ void step_finish(const StepArgs& args, int wslot, Sta
        * (baseEnv.py:54), the reset one is.  Simulate mode: the settle launches that follow rewrite the row. */
       if (valid)
         begin_reset<NJL>(d, sc, D0, e, leg, L.gid, args.seed_lo, args.seed_hi, d.mut[kMutGoalRadius],
-                         args.reset_simulate, -1, st, ln, cforce, goal, potential, bk);
+                         args.reset_simulate, -1, st, ln, cforce, goal, potential, bk, RAND ? dyn : nullptr);
     }
     /* ONE derivation of get_current_state per step, after the reset decision: it is the observation's first
      * block, and the row the next step pushes into the history */
@@ -804,9 +829,12 @@ __device__ __forceinline__ void step_finish(const StepArgs& args, int wslot, Sta
  * substep streams its code from L2, and warps that drift apart each pay for the fetch
  * (profiles/r1_sweep_wpb.txt: +6 % at 4096 envs, +38 % at 64k envs against one warp per block).
  * Eight envs per warp always: narrower warps were measured slower at every size
- * (profiles/r1_sweep_epw.txt). */
-template <int NJL, int MINB, int WPB, bool LIMITS, bool BODY = false>
-__global__ void __launch_bounds__(kBlockThreads * WPB, MINB) step_kernel(const __grid_constant__ StepArgs args) {
+ * (profiles/r1_sweep_epw.txt).
+ * RAND (SoloSimParams.randomize): every lane holds its env's dynamics (EnvDyn) in registers for the launch; the
+ * builds without it are the code of a handle that has never heard of randomisation. */
+template <int NJL, int MINB, int WPB, bool LIMITS, bool BODY = false, bool RAND = false>
+__global__ void __launch_bounds__(kBlockThreads * WPB, MINB) step_kernel(const __grid_constant__ StepArgs args,
+                                                                         const __grid_constant__ DynArgs dyn) {
   __shared__ Smem sm;
   __shared__ __align__(16) StageTile stage[WPB];
   extern __shared__ __align__(16) float body_smem[];   /* BODY: the row records of the block's 8 x WPB envs */
@@ -824,7 +852,7 @@ __global__ void __launch_bounds__(kBlockThreads * WPB, MINB) step_kernel(const _
   const int nsub = (args.mode == MODE_SUBSTEP) ? 1 : sc.frame_skip;
   const int wslot = blockIdx.x * WPB + wib;
   EnvLane<NJL> L;
-  step_load<NJL>(args, wslot, tid, stage[wib], L);
+  step_load<NJL, RAND>(args, wslot, tid, stage[wib], L, &dyn);
   KSTAMP(1);
   for (int s = 0; s < nsub; s++) {                  /* frame_skip x p.stepSimulation() (solo.py:264-265) */
     if (WPB > 1) __syncthreads();   /* keep the warps of a block on the same instruction lines */
@@ -834,10 +862,11 @@ __global__ void __launch_bounds__(kBlockThreads * WPB, MINB) step_kernel(const _
     for (int k = 0; k < NJL; k++) tau_s[k] = torque_on ? L.tau[k] : 0.f;
     group_substep<NJL, LIMITS, BODY>(sm.leg[L.leg], args.mc, sc, L.leg, L.st, L.ln, tau_s, L.cforce, L.bk.nc_sum,
                                      L.bk.sweep_feet, s, nullptr,
-                                     BODY ? body_smem + (size_t)(wib * 8 + L.el) * kBodyEnvStride : nullptr);
+                                     BODY ? body_smem + (size_t)(wib * 8 + L.el) * kBodyEnvStride : nullptr,
+                                     RAND ? &L.dyn : nullptr);
   }
   KSTAMP(2);
-  step_finish<NJL>(args, wslot, stage[wib], L);
+  step_finish<NJL, RAND>(args, wslot, stage[wib], L, &dyn);
   KSTAMP(3);
 }
 
@@ -978,7 +1007,8 @@ __global__ void reset_kernel(const __grid_constant__ ResetArgs args) {
   float cforce;
   EnvBook bk = d.book[e];
   begin_reset<NJL>(d, args.sc, args.D0, e, leg, args.env_id_offset + e, args.seed_lo, args.seed_hi,
-                   d.mut[kMutGoalRadius], args.reset_simulate, args.force_settle, st, ln, cforce, goal, potential, bk);
+                   d.mut[kMutGoalRadius], args.reset_simulate, args.force_settle, st, ln, cforce, goal, potential, bk,
+                   &args.dyn);
   if (!args.reset_simulate) {
     RowPieces<NJL> cur;
     make_pieces<NJL>(args.sc, st, ln, cforce, goal, cur);
@@ -1113,7 +1143,8 @@ __global__ void contacts_kernel(DevArrays d, SimConst sc, int n, float* out) {
 
 /* contact-free forward dynamics on caller-provided states (test hook) */
 template <int NJL>
-__global__ void fd_kernel(ModelConst mc, SimConst sc, int n, const float* state, const float* tau_in, float* out) {
+__global__ void fd_kernel(ModelConst mc, SimConst sc, int n, const float* state, const float* tau_in, float* out,
+                          const float4* envp) {
   __shared__ LegConst sleg[4];
   {
     const float* src = reinterpret_cast<const float*>(&mc.leg[0]);
@@ -1145,7 +1176,9 @@ __global__ void fd_kernel(ModelConst mc, SimConst sc, int n, const float* state,
   sum4_sym6(IA);
 #pragma unroll
   for (int i = 0; i < 6; i++) pA[i] = sum4(pA[i]);
-  base_solve(mc, sc, bw, IA, pA, a0);
+  EnvDyn dyn;
+  if (envp != nullptr) { const float4 p = envp[e]; dyn.mu = p.x; dyn.sm = p.y; dyn.st = p.z; }
+  base_solve(mc, sc, bw, IA, pA, a0, envp != nullptr ? &dyn : nullptr);
   leg_outward<NJL>(ln, a0, qdd);
   base_world_acc(sc, bw, a0, aw, al);
   if (env < n) {
@@ -1157,18 +1190,30 @@ __global__ void fd_kernel(ModelConst mc, SimConst sc, int n, const float* state,
 }
 
 template <int NJL>
-__global__ void torque_kernel(DevArrays d, SimConst sc, int n, int A, const float* actions, float* tau) {
+__global__ void torque_kernel(DevArrays d, SimConst sc, int n, int A, const float* actions, float* tau,
+                              const float4* envp) {
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   const int e = t >> 2, leg = t & 3;
   if (e >= n) return;
   const float* a = actions + (size_t)e * A;
   float kp = sc.kp, kd = sc.kd;
   if (sc.control == 2) { kp = a[4 * NJL]; kd = a[4 * NJL + 1]; }
+  const float st = envp != nullptr ? envp[e].z : 1.f;
 #pragma unroll
   for (int k = 0; k < NJL; k++) {
     float q = d.q[((size_t)k * d.cap + e) * 4 + leg], qd = d.qd[((size_t)k * d.cap + e) * 4 + leg];
-    tau[(size_t)e * 4 * NJL + leg * NJL + k] = action_to_torque(sc, a[leg * NJL + k], q, qd, kp, kd);
+    float t = action_to_torque(sc, a[leg * NJL + k], q, qd, kp, kd);
+    if (envp != nullptr) t *= st;
+    tau[(size_t)e * 4 * NJL + leg * NJL + k] = t;
   }
+}
+
+/* solo_get_env_params: envp [n] float4 -> out [n][3] */
+__global__ void env_params_kernel(const float4* envp, int n, float* out) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= n) return;
+  const float4 p = envp[e];
+  out[3 * e] = p.x; out[3 * e + 1] = p.y; out[3 * e + 2] = p.z;
 }
 
 /* copy env rows 0..K-1 into the reset cache */
@@ -1357,6 +1402,9 @@ struct SoloHandle {
   /* staging for solo_step_host */
   float *s_act, *s_obs, *s_rew, *s_done;
   int host_zero_copy;   /* SOLO_HOST_ZERO_COPY != 0 */
+  /* randomised dynamics: per-env (mu, base mass scale, motor strength, 0), nominal until a reset draws them */
+  int randomize;
+  DynArgs dyn;
 };
 
 static thread_local std::string g_err;
@@ -1388,17 +1436,17 @@ static int grid_min() {
   if (v < 0) { const char* ev = getenv("SOLO_GRID_MIN"); v = ev ? atoi(ev) : 0; }
   return v;
 }
-template <int MINB, int WPB>
+template <int MINB, int WPB, bool RAND>
 static void launch_step_variant(SoloHandle* h, const StepArgs& a, cudaStream_t s) {
   int blocks = (a.n + 8 * WPB - 1) / (8 * WPB);
   if (blocks < grid_min()) blocks = grid_min();
   const bool lim = h->sc.joint_limits != 0;
   if (h->njl == 3) {
-    if (lim) step_kernel<3, MINB, WPB, true><<<blocks, kBlockThreads * WPB, 0, s>>>(a);
-    else step_kernel<3, MINB, WPB, false><<<blocks, kBlockThreads * WPB, 0, s>>>(a);
+    if (lim) step_kernel<3, MINB, WPB, true, false, RAND><<<blocks, kBlockThreads * WPB, 0, s>>>(a, h->dyn);
+    else step_kernel<3, MINB, WPB, false, false, RAND><<<blocks, kBlockThreads * WPB, 0, s>>>(a, h->dyn);
   } else {
-    if (lim) step_kernel<2, MINB, WPB, true><<<blocks, kBlockThreads * WPB, 0, s>>>(a);
-    else step_kernel<2, MINB, WPB, false><<<blocks, kBlockThreads * WPB, 0, s>>>(a);
+    if (lim) step_kernel<2, MINB, WPB, true, false, RAND><<<blocks, kBlockThreads * WPB, 0, s>>>(a, h->dyn);
+    else step_kernel<2, MINB, WPB, false, false, RAND><<<blocks, kBlockThreads * WPB, 0, s>>>(a, h->dyn);
   }
 }
 /* shape of the throughput build: warps per block and resident blocks per SM (the register cap follows:
@@ -1412,21 +1460,23 @@ static void launch_step_variant(SoloHandle* h, const StepArgs& a, cudaStream_t s
 /* body_contacts: the latency shape (4 warps per block) plus the row records in dynamic shared memory */
 constexpr int kBodyWPB = 4;
 constexpr size_t kBodySmemBytes = (size_t)kBodyWPB * 8 * kBodyEnvStride * sizeof(float);
+template <bool RAND>
 static void launch_step_body(SoloHandle* h, const StepArgs& a, cudaStream_t s) {
   int blocks = (a.n + 8 * kBodyWPB - 1) / (8 * kBodyWPB);
   const bool lim = h->sc.joint_limits != 0;
   const int threads = kBlockThreads * kBodyWPB;
   if (h->njl == 3) {
-    if (lim) step_kernel<3, 1, kBodyWPB, true, true><<<blocks, threads, kBodySmemBytes, s>>>(a);
-    else step_kernel<3, 1, kBodyWPB, false, true><<<blocks, threads, kBodySmemBytes, s>>>(a);
+    if (lim) step_kernel<3, 1, kBodyWPB, true, true, RAND><<<blocks, threads, kBodySmemBytes, s>>>(a, h->dyn);
+    else step_kernel<3, 1, kBodyWPB, false, true, RAND><<<blocks, threads, kBodySmemBytes, s>>>(a, h->dyn);
   } else {
-    if (lim) step_kernel<2, 1, kBodyWPB, true, true><<<blocks, threads, kBodySmemBytes, s>>>(a);
-    else step_kernel<2, 1, kBodyWPB, false, true><<<blocks, threads, kBodySmemBytes, s>>>(a);
+    if (lim) step_kernel<2, 1, kBodyWPB, true, true, RAND><<<blocks, threads, kBodySmemBytes, s>>>(a, h->dyn);
+    else step_kernel<2, 1, kBodyWPB, false, true, RAND><<<blocks, threads, kBodySmemBytes, s>>>(a, h->dyn);
   }
 }
 static void launch_step(SoloHandle* h, const StepArgs& a, cudaStream_t s) {
   if (h->sc.body_contacts) {
-    launch_step_body(h, a, s);
+    if (h->randomize) launch_step_body<true>(h, a, s);
+    else launch_step_body<false>(h, a, s);
     h->launches++;
     return;
   }
@@ -1441,8 +1491,13 @@ static void launch_step(SoloHandle* h, const StepArgs& a, cudaStream_t s) {
       if (lim) wide_step_kernel<2, true><<<blocks, kWThreads, sizeof(WideShared), s>>>(a);
       else wide_step_kernel<2, false><<<blocks, kWThreads, sizeof(WideShared), s>>>(a);
     }
-  } else if (h->variant == VARIANT_THROUGHPUT) launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB>(h, a, s);
-  else launch_step_variant<1, 4>(h, a, s);
+  } else if (h->variant == VARIANT_THROUGHPUT) {
+    if (h->randomize) launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB, true>(h, a, s);
+    else launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB, false>(h, a, s);
+  } else {
+    if (h->randomize) launch_step_variant<1, 4, true>(h, a, s);
+    else launch_step_variant<1, 4, false>(h, a, s);
+  }
   h->launches++;
 }
 /* latency build up to 8192 envs (one resident wave of 8 warps per SM), throughput build beyond;
@@ -1464,6 +1519,8 @@ static ResetArgs make_reset_args(SoloHandle* h, int n, const uint8_t* mask, floa
   a.env_id_offset = h->env_id_offset;
   a.reset_simulate = (h->params.reset_mode == SOLO_RESET_SIMULATE);
   a.force_settle = -1;
+  a.dyn = h->dyn;
+  if (!h->randomize) a.dyn.envp = nullptr;
   return a;
 }
 static void launch_reset(SoloHandle* h, const ResetArgs& a, cudaStream_t s) {
@@ -1513,6 +1570,7 @@ int solo_destroy(SoloHandle* h) {
   cudaFree(h->d.rc_base); cudaFree(h->d.rc_q); cudaFree(h->d.rc_qd); cudaFree(h->d.rc_cforce); cudaFree(h->d.rc_hist);
   cudaFree(const_cast<float*>(h->d.mut));
   cudaFree(h->s_act); cudaFree(h->s_obs); cudaFree(h->s_rew); cudaFree(h->s_done);
+  cudaFree(h->dyn.envp);
   delete h;
   return SOLO_OK;
 }
@@ -1535,6 +1593,11 @@ int solo_create(const SoloModelTable* model, const SoloSimParams* params, int32_
   if (rc == SOLO_OK && params->joint_limits && params->limit_rows_per_leg != 1) {
     rc = SOLO_E_ARG; err = "joint_limits: the kernels solve one limit row per leg (limit_rows_per_leg must be 1)";
   }
+  if (rc == SOLO_OK) rc = build_env_ranges(*params, h->dyn.ranges, err);
+  h->randomize = params->randomize ? 1 : 0;
+  if (rc == SOLO_OK && h->randomize && !params->body_contacts && choose_variant(num_envs) == VARIANT_WIDE) {
+    rc = SOLO_E_ARG; err = "randomize: the wide build (SOLO_STEP_VARIANT=wide) has no randomised dynamics";
+  }
   if (rc != SOLO_OK) { delete h; return fail(nullptr, rc, err); }
   h->n = num_envs; h->njl = h->mc.njl; h->nj = 4 * h->njl;
   h->A = h->nj + (params->control == SOLO_CONTROL_VPD ? 2 : 0);
@@ -1547,6 +1610,7 @@ int solo_create(const SoloModelTable* model, const SoloSimParams* params, int32_
   h->K = params->settle_max - params->settle_min; if (h->K < 1) h->K = 1;
   h->cap = num_envs > h->K ? num_envs : h->K;
   h->s_act = h->s_obs = h->s_rew = h->s_done = nullptr;
+  h->dyn.envp = nullptr;
   { const char* ev = getenv("SOLO_HOST_ZERO_COPY"); h->host_zero_copy = !(ev && ev[0] == '0'); }
   memset(&h->d, 0, sizeof(h->d));
   h->d.cap = h->cap;
@@ -1578,6 +1642,10 @@ static int allocate_and_prime(SoloHandle* h, const SoloSimParams* params) {
     CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<3, 1, kBodyWPB, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
     CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<2, 1, kBodyWPB, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
     CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<2, 1, kBodyWPB, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<3, 1, kBodyWPB, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<3, 1, kBodyWPB, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<2, 1, kBodyWPB, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<2, 1, kBodyWPB, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
   }
   const size_t cap = (size_t)h->cap;
   {
@@ -1594,6 +1662,7 @@ static int allocate_and_prime(SoloHandle* h, const SoloSimParams* params) {
   CUDA_TRY(h, cudaMalloc(&h->d.hist, (cap * (H > 0 ? H : 1)) * h->D0 * sizeof(float)));
   CUDA_TRY(h, cudaMalloc(&h->d.fext, cap * 4 * sizeof(float)));
   CUDA_TRY(h, cudaMemset(h->d.fext, 0, cap * 4 * sizeof(float)));
+  CUDA_TRY(h, cudaMalloc(&h->dyn.envp, cap * sizeof(float4)));
   CUDA_TRY(h, cudaMalloc(&h->d.currow, cap * h->D0 * sizeof(float)));
   CUDA_TRY(h, cudaMemset(h->d.currow, 0, cap * h->D0 * sizeof(float)));
   CUDA_TRY(h, cudaMalloc(&h->d.book, cap * sizeof(EnvBook)));
@@ -1640,6 +1709,10 @@ static int allocate_and_prime(SoloHandle* h, const SoloSimParams* params) {
     CUDA_TRY(h, cudaMemsetAsync(h->d.currow, 0, cap * h->D0 * sizeof(float), s));
     CUDA_TRY(h, cudaStreamSynchronize(s));
     CUDA_TRY(h, cudaGetLastError());
+  }
+  {   /* nominal dynamics until the first reset (this also drops what the cache generation drew) */
+    const std::vector<float4> nominal(cap, make_float4(h->sc.mu, 1.f, 1.f, 0.f));
+    CUDA_TRY(h, cudaMemcpy(h->dyn.envp, nominal.data(), cap * sizeof(float4), cudaMemcpyHostToDevice));
   }
   return SOLO_OK;
 }
@@ -1785,8 +1858,9 @@ int solo_forward_dynamics(SoloHandle* h, const float* d_state, const float* d_ta
   if (!h || !d_state || !d_tau || !d_qdd) return fail(h, SOLO_E_ARG, "null argument");
   cudaStream_t s = (cudaStream_t)stream;
   const int threads = 128, blocks = (h->n * 4 + threads - 1) / threads;
-  if (h->njl == 3) fd_kernel<3><<<blocks, threads, 0, s>>>(h->mc, h->sc, h->n, d_state, d_tau, d_qdd);
-  else fd_kernel<2><<<blocks, threads, 0, s>>>(h->mc, h->sc, h->n, d_state, d_tau, d_qdd);
+  const float4* envp = h->randomize ? h->dyn.envp : nullptr;
+  if (h->njl == 3) fd_kernel<3><<<blocks, threads, 0, s>>>(h->mc, h->sc, h->n, d_state, d_tau, d_qdd, envp);
+  else fd_kernel<2><<<blocks, threads, 0, s>>>(h->mc, h->sc, h->n, d_state, d_tau, d_qdd, envp);
   h->launches++;
   CUDA_TRY(h, cudaGetLastError());
   return SOLO_OK;
@@ -1843,8 +1917,17 @@ int solo_action_to_torque(SoloHandle* h, const float* d_actions, float* d_tau, v
   if (!h || !d_actions || !d_tau) return fail(h, SOLO_E_ARG, "null argument");
   cudaStream_t s = (cudaStream_t)stream;
   const int threads = 128, blocks = (h->n * 4 + threads - 1) / threads;
-  if (h->njl == 3) torque_kernel<3><<<blocks, threads, 0, s>>>(h->d, h->sc, h->n, h->A, d_actions, d_tau);
-  else torque_kernel<2><<<blocks, threads, 0, s>>>(h->d, h->sc, h->n, h->A, d_actions, d_tau);
+  const float4* envp = h->randomize ? h->dyn.envp : nullptr;
+  if (h->njl == 3) torque_kernel<3><<<blocks, threads, 0, s>>>(h->d, h->sc, h->n, h->A, d_actions, d_tau, envp);
+  else torque_kernel<2><<<blocks, threads, 0, s>>>(h->d, h->sc, h->n, h->A, d_actions, d_tau, envp);
+  h->launches++;
+  CUDA_TRY(h, cudaGetLastError());
+  return SOLO_OK;
+}
+
+int solo_get_env_params(SoloHandle* h, float* d_out, void* stream) {
+  if (!h || !d_out) return fail(h, SOLO_E_ARG, "null argument");
+  env_params_kernel<<<(h->n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->dyn.envp, h->n, d_out);
   h->launches++;
   CUDA_TRY(h, cudaGetLastError());
   return SOLO_OK;
@@ -1918,8 +2001,10 @@ int solo_debug_wide_trace_helpers(long long* h_out) {
 
 const char* solo_step_variant(const SoloHandle* h) {
   if (!h) return "";
-  if (h->sc.body_contacts) return "body";    /* step_kernel<..., BODY>: the latency shape + the general contact path */
-  return h->variant == VARIANT_WIDE ? "wide" : (h->variant == VARIANT_THROUGHPUT ? "throughput" : "latency");
+  if (h->sc.body_contacts) return h->randomize ? "body+rand" : "body";  /* step_kernel<..., BODY>: the latency shape + the general contact path */
+  if (h->variant == VARIANT_WIDE) return "wide";
+  if (h->variant == VARIANT_THROUGHPUT) return h->randomize ? "throughput+rand" : "throughput";
+  return h->randomize ? "latency+rand" : "latency";
 }
 
 }  // extern "C"

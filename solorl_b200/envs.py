@@ -153,6 +153,11 @@ class SoloVecEnv:
     def get_observation(self):
         return self.sim.get_observation()
 
+    def get_env_params(self):
+        """[N,3] (friction, base_mass_scale, motor_strength) of each env's current episode: privileged inputs
+        for an asymmetric critic, or logging (see the ``randomize_*`` config keys)."""
+        return self.sim.env_params()
+
     def get_torques(self):
         raise NotImplementedError("get_torques is a gait-env call (env.robot.tau_ff)")  # envs.py:45-46
 
@@ -248,6 +253,9 @@ class PyTorchEnvWrapper:
 
     def get_observation(self):
         return self.envs.get_observation()
+
+    def get_env_params(self):
+        return self.envs.get_env_params()
 
     def get_torques(self):
         return self.envs.get_torques()

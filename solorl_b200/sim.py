@@ -119,6 +119,13 @@ class SoloSim:
         d = self._f32(done, (self.n,))
         _lib.check(self.L.solo_accumulate_episode_stats(self.h, _ptr(d), _ptr(acc), self._stream()), self.h)
 
+    def env_params(self):
+        """float32 [N,3] on the device: the (friction, base_mass_scale, motor_strength) each env runs its episode
+        with (drawn at its last reset on a randomised handle, nominal otherwise).  No sync."""
+        out = torch.empty(self.n, 3, dtype=torch.float32, device=self.device)
+        _lib.check(self.L.solo_get_env_params(self.h, _ptr(out), self._stream()), self.h)
+        return out
+
     def set_goal_radius(self, r):
         _lib.check(self.L.solo_set_goal_radius(self.h, float(r)), self.h)
 
