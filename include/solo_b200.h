@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define SOLO_ABI_VERSION 2
+#define SOLO_ABI_VERSION 3
 
 #define SOLO_MAX_LINKS 20
 #define SOLO_MAX_FEET 4
@@ -172,6 +172,21 @@ typedef struct SoloSimParams {
   double friction_lo, friction_hi;
   double base_mass_scale_lo, base_mass_scale_hi;
   double motor_strength_lo, motor_strength_hi;
+  /* Random pushes: a horizontal force on the base, in base axes at the base origin, held as a rectangular pulse
+   * through every substep of push_duration consecutive control steps once in every push_interval control steps.
+   * With t = the env's control steps completed in its episode, j = t / push_interval and r = t % push_interval,
+   * one draw of the env's RNG stream per (episode, j) gives the window's start s in [0, interval - duration] and
+   * the force (fx, fy, 0), fx and fy uniform in [-push_force, push_force]; step t is pushed iff s <= r < s + D.
+   * The schedule starts again at t = 0 with every episode.  Pushes act in the control steps of solo_step /
+   * solo_step_host only: not in the settle steps of a reset (so cached resets stay exact), solo_substep,
+   * solo_forward_dynamics, solo_action_to_torque or solo_actuator_step.  Not available in the wide build.
+   *   push_force     F in N, finite, >= 0;
+   *   push_interval  I in control steps; 0 = pushes off (default), and then the other two are not read;
+   *   push_duration  D in control steps, 1 <= D <= I.
+   * solo_create also rejects episode_length / I >= 2^30. */
+  double push_force;
+  int32_t push_interval;
+  int32_t push_duration;
 } SoloSimParams;
 
 /* Per-env episode record, valid for envs whose `done` was 1 at the last step
@@ -275,6 +290,11 @@ int solo_action_to_torque(SoloHandle* h, const float* d_actions, float* d_tau, v
  * (friction, 1, 1) otherwise and before the first reset. */
 int solo_get_env_params(SoloHandle* h, float* d_out, void* stream);
 
+/* The push the next solo_step applies to each env (SoloSimParams.push_*), d_out float[N, 3] = (fx, fy, 0) in N,
+ * base axes: zero outside a push window and on a handle without pushes.  A pure function of the env's episode
+ * and step count (privileged critic inputs, logging). */
+int solo_get_push_force(SoloHandle* h, float* d_out, void* stream);
+
 /* Gait envs (SURVEY §8f n2): n_ticks simulator ticks under the joint-level PD + feed-forward actuator
  * that the external PyBulletSimulator exposes to baseControlEnv.py:256-270
  * (SetDesiredJointPDgains / Position / Velocity / Torque + SendCommand):
@@ -287,7 +307,8 @@ int solo_actuator_step(SoloHandle* h, const float* d_cmd, int32_t n_ticks, void*
 /* Gait envs: external force on the base for the following solo_actuator_step calls, d_force float[N, 3] in base
  * (link-frame) axes, acting at the base origin -- the random pushes of baseControlEnv.py:276-289, which the
  * external simulator applies with pyb.applyExternalForce(robot, -1, F, [0,0,0], LINK_FRAME) [3P].  Stays in
- * force until overwritten; zero after solo_create.  solo_step / solo_substep ignore it. */
+ * force until overwritten; zero after solo_create.  solo_step / solo_substep ignore it: the RL envs' step has
+ * pushes of its own (SoloSimParams.push_*). */
 int solo_set_external_force(SoloHandle* h, const float* d_force, void* stream);
 
 /* World-frame centres of the four foot collision spheres, d_out float[N, 4, 3]
@@ -322,8 +343,8 @@ int solo_gae(const float* d_rewards, const float* d_values, const float* d_masks
 int64_t solo_launch_count(const SoloHandle* h);
 
 /* Which build of the step kernel this handle launches ("latency", "throughput", "wide", or "body" when
- * SoloSimParams.body_contacts is set; "+rand" appended on a randomised handle): chosen at create time from the
- * batch size, SOLO_STEP_VARIANT overrides (bench / profile evidence). */
+ * SoloSimParams.body_contacts is set; "+rand" appended on a randomised handle, then "+push" on a handle with
+ * pushes): chosen at create time from the batch size, SOLO_STEP_VARIANT overrides (bench / profile evidence). */
 const char* solo_step_variant(const SoloHandle* h);
 
 #ifdef __cplusplus

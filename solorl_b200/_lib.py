@@ -23,7 +23,7 @@ SYMBOLS = [
     "solo_substep", "solo_action_to_torque", "solo_episode_stats", "solo_set_goal_radius",
     "solo_gae", "solo_launch_count", "solo_actuator_step", "solo_get_feet",
     "solo_accumulate_episode_stats", "solo_set_contacts", "solo_step_variant", "solo_set_external_force",
-    "solo_get_env_params",
+    "solo_get_env_params", "solo_get_push_force",
 ]
 
 
@@ -65,6 +65,7 @@ def lib():
     L.solo_substep.argtypes = [vp, fp, vp]
     L.solo_action_to_torque.argtypes = [vp, fp, fp, vp]
     L.solo_get_env_params.argtypes = [vp, fp, vp]
+    L.solo_get_push_force.argtypes = [vp, fp, vp]
     L.solo_episode_stats.argtypes = [vp, fp, vp]
     L.solo_actuator_step.argtypes = [vp, fp, C.c_int32, vp]
     L.solo_get_feet.argtypes = [vp, fp, vp]

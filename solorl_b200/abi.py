@@ -10,7 +10,7 @@ import numpy as np
 
 from .model import SoloModel
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 MAX_LINKS = 20
 MAX_FEET = 4
 
@@ -101,6 +101,9 @@ class SoloSimParams(C.Structure):
         ("base_mass_scale_hi", C.c_double),
         ("motor_strength_lo", C.c_double),
         ("motor_strength_hi", C.c_double),
+        ("push_force", C.c_double),
+        ("push_interval", C.c_int32),
+        ("push_duration", C.c_int32),
     ]
 
 
@@ -217,6 +220,9 @@ def default_params() -> SoloSimParams:
     p.friction_lo = p.friction_hi = 0.0
     p.base_mass_scale_lo = p.base_mass_scale_hi = 0.0
     p.motor_strength_lo = p.motor_strength_hi = 0.0
+    # random pushes off (push_interval = 0); params_from_config sets all three
+    p.push_force = 0.0
+    p.push_interval = p.push_duration = 0
     return p
 
 
@@ -253,6 +259,45 @@ def _randomize_from_config(config: dict, p: SoloSimParams) -> None:
         setattr(p, f_hi, hi)
 
 
+_PUSH_KEYS = ("push_force", "push_interval", "push_duration")
+
+
+def _push_from_config(config: dict, p: SoloSimParams) -> None:
+    """Random pushes: ``push_force`` (N, >= 0), ``push_interval`` and ``push_duration`` (control steps,
+    ``1 <= push_duration <= push_interval``).  ``push_force`` turns pushes on and needs the other two; a missing
+    key or a malformed value raises ``ValueError``."""
+    present = [k for k in _PUSH_KEYS if k in config]
+    if not present:
+        return
+    if len(present) != len(_PUSH_KEYS):
+        missing = [k for k in _PUSH_KEYS if k not in config]
+        raise ValueError(f"random pushes need all of {', '.join(_PUSH_KEYS)}; missing {', '.join(missing)}")
+    try:
+        force = float(config["push_force"])
+    except (TypeError, ValueError):
+        raise ValueError(f"push_force must be a number, got {config['push_force']!r}") from None
+    if not (np.isfinite(force) and force >= 0):
+        raise ValueError(f"push_force must be finite and >= 0, got {force}")
+    steps = {}
+    for k in ("push_interval", "push_duration"):
+        try:
+            v = float(config[k])
+        except (TypeError, ValueError):
+            v = float("nan")
+        if not (np.isfinite(v) and v == int(v)):
+            raise ValueError(f"{k} must be a whole number of control steps, got {config[k]!r}")
+        steps[k] = int(v)
+    interval, duration = steps["push_interval"], steps["push_duration"]
+    if interval < 1:
+        raise ValueError(f"push_interval must be >= 1 when push_force is set, got {interval}")
+    if not 1 <= duration <= interval:
+        raise ValueError(f"push_duration must satisfy 1 <= push_duration <= push_interval ({interval}), "
+                         f"got {duration}")
+    if p.episode_length // interval >= 2 ** 30:
+        raise ValueError("episode_length / push_interval must be below 2^30")
+    p.push_force, p.push_interval, p.push_duration = force, interval, duration
+
+
 def params_from_config(config: dict, model: Optional[SoloModel] = None) -> SoloSimParams:
     """Map a reference config dict onto ``SoloSimParams``.
 
@@ -262,7 +307,8 @@ def params_from_config(config: dict, model: Optional[SoloModel] = None) -> SoloS
     ``use_treadmill`` False.  Extra keys (all default to the reference-faithful value):
     ``torque_hold``, ``solver_iters``, ``solver_residual_threshold``, ``contact_erp``, ``reset_mode``;
     ``randomize_friction``, ``randomize_base_mass``, ``randomize_motor_strength`` (per-env randomised
-    dynamics, see ``_randomize_from_config``).
+    dynamics, see ``_randomize_from_config``); ``push_force``, ``push_interval``, ``push_duration`` (random
+    pushes on the base, see ``_push_from_config``).
     """
     p = default_params()
     p.episode_length = int(config["episode_length"])           # baseEnv.py:164 (required)
@@ -304,6 +350,7 @@ def params_from_config(config: dict, model: Optional[SoloModel] = None) -> SoloS
     rm = config.get("reset_mode", "cached")
     p.reset_mode = {"cached": RESET_CACHED, "simulate": RESET_SIMULATE}[rm]
     _randomize_from_config(config, p)
+    _push_from_config(config, p)
     return p
 
 

@@ -122,9 +122,12 @@ struct EnvRanges {
   float mu_lo, mu_hi, sm_lo, sm_hi, st_lo, st_hi;
 };
 
-/* Philox draw index of the dynamics draw: the per-episode draws (settle count and goal at the reset, new goals while
- * stepping) count up from 0 and never reach it, so they stay what they are without randomisation. */
+/* Philox draw indices of the dynamics draw and of the push draws: the per-episode draws (settle count and goal at
+ * the reset, new goals while stepping) count up from 0 and never reach kDynDraw; the push draw of interval j is
+ * kPushDraw + j, and solo_create keeps j below 2^30, so it never reaches back to kDynDraw or wraps to 0.  Every
+ * draw therefore stays what it is without randomisation or pushes. */
 constexpr uint32_t kDynDraw = 0x80000000u;
+constexpr uint32_t kPushDraw = 0xC0000000u;
 
 /* The dynamics of env `gid` for episode `episode`: each value uniform in its range.  fmaf keeps the device and a
  * host replay bit-identical; fminf keeps a rounded-up product inside the range. */
@@ -139,6 +142,36 @@ SOLO_HD EnvDyn sample_env_dyn(const EnvRanges& r, uint32_t seed_lo, uint32_t see
   p.sm = dyn_uniform(r.sm_lo, r.sm_hi, w[1]);
   p.st = dyn_uniform(r.st_lo, r.st_hi, w[2]);
   return p;
+}
+
+/* Random pushes (SoloSimParams.push_*, narrowed to float / int): interval 0 = off. */
+struct PushParams {
+  float force;
+  int32_t interval, duration;
+};
+struct PushSample {
+  bool on;
+  float fx, fy;   /* base axes; 0 when !on */
+};
+
+/* The push of env `gid` in control step t (steps completed in episode `episode`): interval j = t / I draws the
+ * window start s = w[0] % (I - D + 1) and the force from one Philox block; step t is pushed iff s <= t % I < s + D. */
+SOLO_HD PushSample sample_push(const PushParams& pp, uint32_t seed_lo, uint32_t seed_hi, long long gid,
+                               uint32_t episode, int32_t t) {
+  PushSample ps;
+  ps.on = false; ps.fx = 0.f; ps.fy = 0.f;
+  if (pp.interval <= 0) return ps;
+  const uint32_t I = (uint32_t)pp.interval, j = (uint32_t)t / I, r = (uint32_t)t % I;
+  uint32_t w[4] = {(uint32_t)((unsigned long long)gid & 0xffffffffull), (uint32_t)((unsigned long long)gid >> 32),
+                   episode, kPushDraw + j};
+  philox4x32_10(w, seed_lo, seed_hi);
+  const uint32_t s = w[0] % (I - (uint32_t)pp.duration + 1u);
+  if (s <= r && r < s + (uint32_t)pp.duration) {
+    ps.on = true;
+    ps.fx = dyn_uniform(-pp.force, pp.force, w[1]);
+    ps.fy = dyn_uniform(-pp.force, pp.force, w[2]);
+  }
+  return ps;
 }
 
 /* robot_specific_reset (solo.py:291-296): base -> (0,0,initial_z), identity, zero velocity */

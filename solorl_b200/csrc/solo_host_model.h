@@ -148,6 +148,25 @@ inline int build_env_ranges(const SoloSimParams& p, EnvRanges& r, std::string& e
   return SOLO_OK;
 }
 
+/* Random pushes, checked when push_interval > 0 (and left 0 otherwise).  episode_length / interval < 2^30 keeps
+ * the push draw index kPushDraw + j from wrapping. */
+inline int build_push_params(const SoloSimParams& p, PushParams& pp, std::string& err) {
+  memset(&pp, 0, sizeof(pp));
+  if (!(isfinite(p.push_force) && p.push_force >= 0)) {
+    err = "push: push_force must be finite and >= 0"; return SOLO_E_ARG;
+  }
+  if (p.push_interval < 0) { err = "push: push_interval must be >= 0 (0 = pushes off)"; return SOLO_E_ARG; }
+  if (p.push_interval == 0) return SOLO_OK;
+  if (p.push_duration < 1 || p.push_duration > p.push_interval) {
+    err = "push: push_duration must satisfy 1 <= push_duration <= push_interval"; return SOLO_E_ARG;
+  }
+  if (p.episode_length / p.push_interval >= (1 << 30)) {
+    err = "push: episode_length / push_interval must be below 2^30"; return SOLO_E_ARG;
+  }
+  pp.force = (float)p.push_force; pp.interval = p.push_interval; pp.duration = p.push_duration;
+  return SOLO_OK;
+}
+
 inline void fill_default_params(SoloSimParams* p) {
   memset(p, 0, sizeof(*p));
   p->abi_version = SOLO_ABI_VERSION;

@@ -85,10 +85,12 @@ struct StepArgs {
 
 /* Randomised dynamics of a handle: per-env (mu, base mass scale, motor strength, 0) and the ranges a reset draws
  * them from; envp == nullptr: randomisation off.  A kernel parameter of its own, after StepArgs, so that the
- * kernels without randomisation keep their parameter layout. */
+ * kernels without randomisation keep their parameter layout.  push: the random pushes (interval 0 = off), last
+ * so that nothing before it moves. */
 struct DynArgs {
   float4* envp;
   EnvRanges ranges;
+  PushParams push;
 };
 
 struct ResetArgs {
@@ -644,7 +646,7 @@ typedef float StageTile[8][kStageD];
 
 /* Step prologue of one lane: state load, apply_action (solo.py:224-259), history push (solo.py:262).
  * wslot = index of this lane's warp among the env warps of the grid (eight envs per warp). */
-template <int NJL, bool RAND = false>
+template <int NJL, bool RAND = false, bool PUSH = false>
 __device__ __forceinline__ void step_load(const StepArgs& args, int wslot, int tid, StageTile& stage, EnvLane<NJL>& L,
                                           const DynArgs* dyn = nullptr) {
   const SimConst& sc = args.sc;
@@ -667,7 +669,7 @@ __device__ __forceinline__ void step_load(const StepArgs& args, int wslot, int t
   L.active = L.valid && (args.mode != MODE_SETTLE || L.bk.settle_left > 0);
   if (RAND) {
     /* the settle steps of a reset run with the nominal dynamics, so that a cached reset stays exact */
-    if (args.mode == MODE_SETTLE) { L.dyn.mu = sc.mu; L.dyn.sm = 1.f; L.dyn.st = 1.f; }
+    if (args.mode == MODE_SETTLE || (PUSH && dyn->envp == nullptr)) { L.dyn.mu = sc.mu; L.dyn.sm = 1.f; L.dyn.st = 1.f; }
     else { const float4 p = dyn->envp[e]; L.dyn.mu = p.x; L.dyn.sm = p.y; L.dyn.st = p.z; }
   }
 #pragma unroll
@@ -698,6 +700,19 @@ __device__ __forceinline__ void step_load(const StepArgs& args, int wslot, int t
   } else if (args.mode == MODE_SUBSTEP) {
 #pragma unroll
     for (int k = 0; k < NJL; k++) L.tau[k] = args.in[(size_t)e * 4 * NJL + leg * NJL + k];
+  }
+  if (PUSH) {
+    /* The env's push for this launch, held in its row of the warp's stage (idle until step_finish writes the
+     * observation rows) rather than in registers.  Pushes act in the control steps only: the settle steps
+     * (cached resets stay exact) and the substep hook run unpushed.  t = the steps this episode has completed,
+     * before step_finish counts this one. */
+    if (leg == 0) {
+      PushSample ps;
+      ps.fx = 0.f; ps.fy = 0.f;
+      if (args.mode == MODE_STEP) ps = sample_push(dyn->push, args.seed_lo, args.seed_hi, L.gid, L.bk.episode, L.bk.timestep);
+      stage[L.el][0] = ps.fx; stage[L.el][1] = ps.fy; stage[L.el][2] = 0.f;
+    }
+    __syncwarp();
   }
   if (args.mode != MODE_SUBSTEP && L.active && sc.H > 0) {   /* simulator_step: history push (solo.py:262) */
     RowPieces<NJL> cur;
@@ -831,8 +846,11 @@ __device__ __forceinline__ void step_finish(const StepArgs& args, int wslot, Sta
  * Eight envs per warp always: narrower warps were measured slower at every size
  * (profiles/r1_sweep_epw.txt).
  * RAND (SoloSimParams.randomize): every lane holds its env's dynamics (EnvDyn) in registers for the launch; the
- * builds without it are the code of a handle that has never heard of randomisation. */
-template <int NJL, int MINB, int WPB, bool LIMITS, bool BODY = false, bool RAND = false>
+ * builds without it are the code of a handle that has never heard of randomisation.
+ * PUSH (SoloSimParams.push_interval > 0), instantiated with RAND only: step_load puts the env's push for the
+ * launch into the warp's stage, and every substep reads it from there as the external force on the base; a handle
+ * with pushes and without randomisation passes envp == nullptr and runs the nominal dynamics. */
+template <int NJL, int MINB, int WPB, bool LIMITS, bool BODY = false, bool RAND = false, bool PUSH = false>
 __global__ void __launch_bounds__(kBlockThreads * WPB, MINB) step_kernel(const __grid_constant__ StepArgs args,
                                                                          const __grid_constant__ DynArgs dyn) {
   __shared__ Smem sm;
@@ -852,7 +870,7 @@ __global__ void __launch_bounds__(kBlockThreads * WPB, MINB) step_kernel(const _
   const int nsub = (args.mode == MODE_SUBSTEP) ? 1 : sc.frame_skip;
   const int wslot = blockIdx.x * WPB + wib;
   EnvLane<NJL> L;
-  step_load<NJL, RAND>(args, wslot, tid, stage[wib], L, &dyn);
+  step_load<NJL, RAND, PUSH>(args, wslot, tid, stage[wib], L, &dyn);
   KSTAMP(1);
   for (int s = 0; s < nsub; s++) {                  /* frame_skip x p.stepSimulation() (solo.py:264-265) */
     if (WPB > 1) __syncthreads();   /* keep the warps of a block on the same instruction lines */
@@ -861,11 +879,12 @@ __global__ void __launch_bounds__(kBlockThreads * WPB, MINB) step_kernel(const _
 #pragma unroll
     for (int k = 0; k < NJL; k++) tau_s[k] = torque_on ? L.tau[k] : 0.f;
     group_substep<NJL, LIMITS, BODY>(sm.leg[L.leg], args.mc, sc, L.leg, L.st, L.ln, tau_s, L.cforce, L.bk.nc_sum,
-                                     L.bk.sweep_feet, s, nullptr,
+                                     L.bk.sweep_feet, s, PUSH ? &stage[wib][L.el][0] : nullptr,
                                      BODY ? body_smem + (size_t)(wib * 8 + L.el) * kBodyEnvStride : nullptr,
                                      RAND ? &L.dyn : nullptr);
   }
   KSTAMP(2);
+  if (PUSH) __syncwarp();                           /* every lane has read the push before the stage is reused */
   step_finish<NJL, RAND>(args, wslot, stage[wib], L, &dyn);
   KSTAMP(3);
 }
@@ -1216,6 +1235,16 @@ __global__ void env_params_kernel(const float4* envp, int n, float* out) {
   out[3 * e] = p.x; out[3 * e + 1] = p.y; out[3 * e + 2] = p.z;
 }
 
+/* solo_get_push_force: the push of each env's next control step, from its episode record -> out [n][3] */
+__global__ void push_force_kernel(const EnvBook* book, PushParams pp, uint32_t seed_lo, uint32_t seed_hi,
+                                  long long env_id_offset, int n, float* out) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= n) return;
+  const EnvBook bk = book[e];
+  const PushSample ps = sample_push(pp, seed_lo, seed_hi, env_id_offset + e, bk.episode, bk.timestep);
+  out[3 * e] = ps.fx; out[3 * e + 1] = ps.fy; out[3 * e + 2] = 0.f;
+}
+
 /* copy env rows 0..K-1 into the reset cache */
 template <int NJL>
 __global__ void fill_cache_kernel(DevArrays d, int K, int H, int D0) {
@@ -1405,6 +1434,7 @@ struct SoloHandle {
   /* randomised dynamics: per-env (mu, base mass scale, motor strength, 0), nominal until a reset draws them */
   int randomize;
   DynArgs dyn;
+  int push;        /* random pushes on (push_interval > 0): the step launches the PUSH builds */
 };
 
 static thread_local std::string g_err;
@@ -1436,17 +1466,25 @@ static int grid_min() {
   if (v < 0) { const char* ev = getenv("SOLO_GRID_MIN"); v = ev ? atoi(ev) : 0; }
   return v;
 }
-template <int MINB, int WPB, bool RAND>
+/* the DynArgs of a launch: envp only on a randomised handle (a handle with pushes alone runs the nominal
+ * dynamics, and its resets draw nothing) */
+static DynArgs dyn_args(const SoloHandle* h) {
+  DynArgs a = h->dyn;
+  if (!h->randomize) a.envp = nullptr;
+  return a;
+}
+template <int MINB, int WPB, bool RAND, bool PUSH = false>
 static void launch_step_variant(SoloHandle* h, const StepArgs& a, cudaStream_t s) {
   int blocks = (a.n + 8 * WPB - 1) / (8 * WPB);
   if (blocks < grid_min()) blocks = grid_min();
   const bool lim = h->sc.joint_limits != 0;
+  const DynArgs dyn = dyn_args(h);
   if (h->njl == 3) {
-    if (lim) step_kernel<3, MINB, WPB, true, false, RAND><<<blocks, kBlockThreads * WPB, 0, s>>>(a, h->dyn);
-    else step_kernel<3, MINB, WPB, false, false, RAND><<<blocks, kBlockThreads * WPB, 0, s>>>(a, h->dyn);
+    if (lim) step_kernel<3, MINB, WPB, true, false, RAND, PUSH><<<blocks, kBlockThreads * WPB, 0, s>>>(a, dyn);
+    else step_kernel<3, MINB, WPB, false, false, RAND, PUSH><<<blocks, kBlockThreads * WPB, 0, s>>>(a, dyn);
   } else {
-    if (lim) step_kernel<2, MINB, WPB, true, false, RAND><<<blocks, kBlockThreads * WPB, 0, s>>>(a, h->dyn);
-    else step_kernel<2, MINB, WPB, false, false, RAND><<<blocks, kBlockThreads * WPB, 0, s>>>(a, h->dyn);
+    if (lim) step_kernel<2, MINB, WPB, true, false, RAND, PUSH><<<blocks, kBlockThreads * WPB, 0, s>>>(a, dyn);
+    else step_kernel<2, MINB, WPB, false, false, RAND, PUSH><<<blocks, kBlockThreads * WPB, 0, s>>>(a, dyn);
   }
 }
 /* shape of the throughput build: warps per block and resident blocks per SM (the register cap follows:
@@ -1460,22 +1498,25 @@ static void launch_step_variant(SoloHandle* h, const StepArgs& a, cudaStream_t s
 /* body_contacts: the latency shape (4 warps per block) plus the row records in dynamic shared memory */
 constexpr int kBodyWPB = 4;
 constexpr size_t kBodySmemBytes = (size_t)kBodyWPB * 8 * kBodyEnvStride * sizeof(float);
-template <bool RAND>
+template <bool RAND, bool PUSH = false>
 static void launch_step_body(SoloHandle* h, const StepArgs& a, cudaStream_t s) {
   int blocks = (a.n + 8 * kBodyWPB - 1) / (8 * kBodyWPB);
   const bool lim = h->sc.joint_limits != 0;
   const int threads = kBlockThreads * kBodyWPB;
+  const DynArgs dyn = dyn_args(h);
   if (h->njl == 3) {
-    if (lim) step_kernel<3, 1, kBodyWPB, true, true, RAND><<<blocks, threads, kBodySmemBytes, s>>>(a, h->dyn);
-    else step_kernel<3, 1, kBodyWPB, false, true, RAND><<<blocks, threads, kBodySmemBytes, s>>>(a, h->dyn);
+    if (lim) step_kernel<3, 1, kBodyWPB, true, true, RAND, PUSH><<<blocks, threads, kBodySmemBytes, s>>>(a, dyn);
+    else step_kernel<3, 1, kBodyWPB, false, true, RAND, PUSH><<<blocks, threads, kBodySmemBytes, s>>>(a, dyn);
   } else {
-    if (lim) step_kernel<2, 1, kBodyWPB, true, true, RAND><<<blocks, threads, kBodySmemBytes, s>>>(a, h->dyn);
-    else step_kernel<2, 1, kBodyWPB, false, true, RAND><<<blocks, threads, kBodySmemBytes, s>>>(a, h->dyn);
+    if (lim) step_kernel<2, 1, kBodyWPB, true, true, RAND, PUSH><<<blocks, threads, kBodySmemBytes, s>>>(a, dyn);
+    else step_kernel<2, 1, kBodyWPB, false, true, RAND, PUSH><<<blocks, threads, kBodySmemBytes, s>>>(a, dyn);
   }
 }
+/* builds: PUSH only with RAND (a handle with pushes and nominal dynamics passes envp == nullptr) */
 static void launch_step(SoloHandle* h, const StepArgs& a, cudaStream_t s) {
   if (h->sc.body_contacts) {
-    if (h->randomize) launch_step_body<true>(h, a, s);
+    if (h->push) launch_step_body<true, true>(h, a, s);
+    else if (h->randomize) launch_step_body<true>(h, a, s);
     else launch_step_body<false>(h, a, s);
     h->launches++;
     return;
@@ -1492,10 +1533,12 @@ static void launch_step(SoloHandle* h, const StepArgs& a, cudaStream_t s) {
       else wide_step_kernel<2, false><<<blocks, kWThreads, sizeof(WideShared), s>>>(a);
     }
   } else if (h->variant == VARIANT_THROUGHPUT) {
-    if (h->randomize) launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB, true>(h, a, s);
+    if (h->push) launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB, true, true>(h, a, s);
+    else if (h->randomize) launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB, true>(h, a, s);
     else launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB, false>(h, a, s);
   } else {
-    if (h->randomize) launch_step_variant<1, 4, true>(h, a, s);
+    if (h->push) launch_step_variant<1, 4, true, true>(h, a, s);
+    else if (h->randomize) launch_step_variant<1, 4, true>(h, a, s);
     else launch_step_variant<1, 4, false>(h, a, s);
   }
   h->launches++;
@@ -1519,8 +1562,7 @@ static ResetArgs make_reset_args(SoloHandle* h, int n, const uint8_t* mask, floa
   a.env_id_offset = h->env_id_offset;
   a.reset_simulate = (h->params.reset_mode == SOLO_RESET_SIMULATE);
   a.force_settle = -1;
-  a.dyn = h->dyn;
-  if (!h->randomize) a.dyn.envp = nullptr;
+  a.dyn = dyn_args(h);
   return a;
 }
 static void launch_reset(SoloHandle* h, const ResetArgs& a, cudaStream_t s) {
@@ -1598,6 +1640,11 @@ int solo_create(const SoloModelTable* model, const SoloSimParams* params, int32_
   if (rc == SOLO_OK && h->randomize && !params->body_contacts && choose_variant(num_envs) == VARIANT_WIDE) {
     rc = SOLO_E_ARG; err = "randomize: the wide build (SOLO_STEP_VARIANT=wide) has no randomised dynamics";
   }
+  if (rc == SOLO_OK) rc = build_push_params(*params, h->dyn.push, err);
+  h->push = params->push_interval > 0 ? 1 : 0;
+  if (rc == SOLO_OK && h->push && !params->body_contacts && choose_variant(num_envs) == VARIANT_WIDE) {
+    rc = SOLO_E_ARG; err = "push: the wide build (SOLO_STEP_VARIANT=wide) has no random pushes";
+  }
   if (rc != SOLO_OK) { delete h; return fail(nullptr, rc, err); }
   h->n = num_envs; h->njl = h->mc.njl; h->nj = 4 * h->njl;
   h->A = h->nj + (params->control == SOLO_CONTROL_VPD ? 2 : 0);
@@ -1646,6 +1693,10 @@ static int allocate_and_prime(SoloHandle* h, const SoloSimParams* params) {
     CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<3, 1, kBodyWPB, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
     CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<2, 1, kBodyWPB, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
     CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<2, 1, kBodyWPB, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<3, 1, kBodyWPB, true, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<3, 1, kBodyWPB, false, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<2, 1, kBodyWPB, true, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    CUDA_TRY(h, cudaFuncSetAttribute(step_kernel<2, 1, kBodyWPB, false, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
   }
   const size_t cap = (size_t)h->cap;
   {
@@ -1933,6 +1984,16 @@ int solo_get_env_params(SoloHandle* h, float* d_out, void* stream) {
   return SOLO_OK;
 }
 
+int solo_get_push_force(SoloHandle* h, float* d_out, void* stream) {
+  if (!h || !d_out) return fail(h, SOLO_E_ARG, "null argument");
+  push_force_kernel<<<(h->n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
+      h->d.book, h->dyn.push, (uint32_t)(h->seed & 0xffffffffu), (uint32_t)(h->seed >> 32), h->env_id_offset, h->n,
+      d_out);
+  h->launches++;
+  CUDA_TRY(h, cudaGetLastError());
+  return SOLO_OK;
+}
+
 int solo_episode_stats(SoloHandle* h, SoloEpisodeStats* d_stats, void* stream) {
   if (!h || !d_stats) return fail(h, SOLO_E_ARG, "null argument");
   CUDA_TRY(h, cudaMemcpyAsync(d_stats, h->d.stats, (size_t)h->n * sizeof(SoloEpisodeStats),
@@ -2001,10 +2062,14 @@ int solo_debug_wide_trace_helpers(long long* h_out) {
 
 const char* solo_step_variant(const SoloHandle* h) {
   if (!h) return "";
-  if (h->sc.body_contacts) return h->randomize ? "body+rand" : "body";  /* step_kernel<..., BODY>: the latency shape + the general contact path */
+  static const char* const kNames[3][4] = {
+      {"latency", "latency+rand", "latency+push", "latency+rand+push"},
+      {"throughput", "throughput+rand", "throughput+push", "throughput+rand+push"},
+      {"body", "body+rand", "body+push", "body+rand+push"}};   /* body: the latency shape + the general contact path */
+  const int opts = (h->randomize ? 1 : 0) + (h->push ? 2 : 0);
+  if (h->sc.body_contacts) return kNames[2][opts];
   if (h->variant == VARIANT_WIDE) return "wide";
-  if (h->variant == VARIANT_THROUGHPUT) return h->randomize ? "throughput+rand" : "throughput";
-  return h->randomize ? "latency+rand" : "latency";
+  return kNames[h->variant == VARIANT_THROUGHPUT ? 1 : 0][opts];
 }
 
 }  // extern "C"

@@ -158,6 +158,11 @@ class SoloVecEnv:
         for an asymmetric critic, or logging (see the ``randomize_*`` config keys)."""
         return self.sim.env_params()
 
+    def get_push_force(self):
+        """[N,3] push (fx, fy, 0) in N, base axes, that the next step applies to each env: privileged inputs for
+        an asymmetric critic, or logging (see the ``push_*`` config keys)."""
+        return self.sim.push_force()
+
     def get_torques(self):
         raise NotImplementedError("get_torques is a gait-env call (env.robot.tau_ff)")  # envs.py:45-46
 
@@ -256,6 +261,9 @@ class PyTorchEnvWrapper:
 
     def get_env_params(self):
         return self.envs.get_env_params()
+
+    def get_push_force(self):
+        return self.envs.get_push_force()
 
     def get_torques(self):
         return self.envs.get_torques()

@@ -126,6 +126,13 @@ class SoloSim:
         _lib.check(self.L.solo_get_env_params(self.h, _ptr(out), self._stream()), self.h)
         return out
 
+    def push_force(self):
+        """float32 [N,3] on the device: the push (fx, fy, 0) in N, base axes, that the next step applies to each
+        env (zero outside a push window and without pushes).  No sync."""
+        out = torch.empty(self.n, 3, dtype=torch.float32, device=self.device)
+        _lib.check(self.L.solo_get_push_force(self.h, _ptr(out), self._stream()), self.h)
+        return out
+
     def set_goal_radius(self, r):
         _lib.check(self.L.solo_set_goal_radius(self.h, float(r)), self.h)
 
