@@ -879,31 +879,40 @@ SOLO_HD void pgs_normal_commit(PL& pl, float nv) {
   pl.lam[0] = nv;
   pl.nl0 = -nv;
 }
-/* candidates for this lane's friction pair (cone) */
-template <class PL>
-SOLO_HD void pgs_cone_candidate(const PL& pl, float mu, float& nA, float& nB, float& dA, float& dB,
-                                float& rv) {
+/* candidates of one friction pair (cone) from the state of its two rows: candidates sA, sB, impulses lA, lB,
+ * diagonals dgA, dgB; lamn = the foot's normal impulse */
+SOLO_HD void cone_candidate(float mu, float lamn, float sA, float sB, float lA, float lB, float dgA, float dgB,
+                            float& nA, float& nB, float& dA, float& dB, float& rv) {
   /* Bullet clamps sA to +-|lim sin(atan2(sA,sB))| and sB to +-|lim cos(.)|, i.e. it scales the pair
    * (sA,sB) back onto the circle of radius lim when it lies outside: (sA,sB) * min(1, lim/|s|).
    * Written for the shortest dependent chain from g to the impulse change: the 1e-30 guard rides in
    * the first FMA instead of a max, and d = s*scale - lambda is one FMA instead of multiply + subtract. */
-  const float lim = mu * pl.lam[0];
-  const float sA = pl.g[1], sB = pl.g[2];
+  const float lim = mu * lamn;
   const float n2 = fmaf(sB, sB, fmaf(sA, sA, 1e-30f));
   const float sc = fminf(lim * solo_rsqrt(n2), 1.0f);
   nA = sA * sc;
   nB = sB * sc;
-  dA = fmaf(sA, sc, -pl.lam[1]);
-  dB = fmaf(sB, sc, -pl.lam[2]);
-  rv = dA * pl.diag[1] + dB * pl.diag[2];
+  dA = fmaf(sA, sc, -lA);
+  dB = fmaf(sB, sc, -lB);
+  rv = dA * dgA + dB * dgB;
+}
+/* candidate of one friction row (pyramid): candidate s, impulse l, diagonal dg */
+SOLO_HD void pyramid_candidate(float mu, float lamn, float s, float l, float dg, float& nv, float& d, float& rv) {
+  const float lim = mu * lamn;
+  nv = clampf(s, -lim, lim);
+  d = nv - l;
+  rv = d * dg;
+}
+/* candidates for this lane's friction pair (cone) */
+template <class PL>
+SOLO_HD void pgs_cone_candidate(const PL& pl, float mu, float& nA, float& nB, float& dA, float& dB,
+                                float& rv) {
+  cone_candidate(mu, pl.lam[0], pl.g[1], pl.g[2], pl.lam[1], pl.lam[2], pl.diag[1], pl.diag[2], nA, nB, dA, dB, rv);
 }
 /* candidate for one friction row (pyramid), q = 0/1 */
 template <class PL>
 SOLO_HD void pgs_pyramid_candidate(const PL& pl, float mu, int q, float& nv, float& d, float& rv) {
-  const float lim = mu * pl.lam[0];
-  nv = clampf(pl.g[1 + q], -lim, lim);
-  d = nv - pl.lam[1 + q];
-  rv = d * pl.diag[1 + q];
+  pyramid_candidate(mu, pl.lam[0], pl.g[1 + q], pl.lam[1 + q], pl.diag[1 + q], nv, d, rv);
 }
 /* Apply the impulse change d of global row `col` to this lane's rows: g[m] += (-B[m][col]) d, B being stored negated.
  * On the GPU two rows go through ONE packed FFMA2 (sm_100 fma.rn.f32x2, the scalar d broadcast by the instruction's

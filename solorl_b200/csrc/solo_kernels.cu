@@ -431,6 +431,233 @@ __device__ __forceinline__ void pgs_sweeps4(PgsLane4& pl, const SimConst& sc, in
   }
 }
 
+/* pgs_sweeps4 with the 16 rows of an env on its four lanes by their position in the sweep, not by foot:
+ *   lane 0: the four limit rows             (slot s: leg kLimLeg[s])
+ *   lane 1: the four normal rows            (slot s: foot kNrmFoot[s])
+ *   lane 2: the friction pairs of feet 0, 1 (slots 2p, 2p+1: rows A, B of foot p)
+ *   lane 3: the friction pairs of feet 2, 3 (slots 2p, 2p+1: rows A, B of foot 2 + p)
+ * so that the sweep's dependent chain changes lanes four times (limit -> normal -> friction of feet 0, 1 -> friction
+ * of feet 2, 3 -> next sweep) instead of nine.  A phase is the run of relaxations of one lane.  Inside it the owner
+ * takes each impulse change at once into a scratch copy of those of its rows that a later relaxation of the phase
+ * reads, from its own value, so that its chain never waits for a shuffle; the changes go to the other lanes by
+ * shuffles issued as each one exists.  At the hand-over to the next phase every lane -- the owner too -- applies the
+ * phase's changes to its rows in sweep order from the shuffled values: on the owner those are the FMAs of its
+ * scratch copy again, same operands, same bits.  Every row thus receives the same FMAs in the same order as with
+ * one lane per foot (pgs_sweeps4), and the result is bit-identical to it.  The slot orders of lanes 0 and 1 follow
+ * from the exchange schedule of pgs_rows_exchange4.
+ * It issues more instructions per sweep than pgs_sweeps4 (limit candidates on one lane, the owner's scratch FMAs, the
+ * normal impulses sent to the friction lanes) for a shorter chain: faster where one env's chain bounds the launch
+ * (latency build, 4096 envs), slower where issue slots do (throughput build, 65 536 envs); see PHASED of step_kernel. */
+struct PgsRows4 {
+  float B[4][kRowsL];   /* negated, scaled Delassus rows (PgsLaneT) */
+  float g[4], diag[4];
+  float x[4];           /* -lambda on lanes 0 and 1 (the h-rows' lower bound of the impulse change), lambda on 2, 3 */
+};
+__device__ constexpr int kLimLeg[4] = {1, 3, 0, 2};
+__device__ constexpr int kNrmFoot[4] = {3, 1, 2, 0};   /* its own inverse */
+/* Exchange schedule between the foot layout (lane = foot; row m: 0 normal, 1 and 2 friction, 3 limit) and the
+ * sweep layout: in round k lane L receives its slot k from lane kXchSrc[k][L], which sends its row kXchRow[k][src]
+ * (kXchDst[k][src] = L is the way back).  Each round is a permutation of the four lanes, so one shuffle per value
+ * and round moves a whole row; rounds 0 and 2 move friction rows A, rounds 1 and 3 rows B. */
+constexpr unsigned xch_pack(int a, int b, int c, int d) { return (unsigned)(a | (b << 2) | (c << 4) | (d << 6)); }
+constexpr unsigned kXchSrc = xch_pack(1, 3, 0, 2) | xch_pack(3, 1, 0, 2) << 8 | xch_pack(0, 2, 1, 3) << 16 |
+                             xch_pack(2, 0, 1, 3) << 24;
+constexpr unsigned kXchDst = xch_pack(2, 0, 3, 1) | xch_pack(2, 1, 3, 0) << 8 | xch_pack(0, 2, 1, 3) << 16 |
+                             xch_pack(1, 2, 0, 3) << 24;
+constexpr unsigned kXchRow = xch_pack(1, 3, 1, 0) | xch_pack(2, 0, 2, 3) << 8 | xch_pack(3, 1, 0, 1) << 16 |
+                             xch_pack(0, 2, 3, 2) << 24;
+__device__ __forceinline__ unsigned xch_field(unsigned table, int k, int leg) { return (table >> (8 * k + 2 * leg)) & 3u; }
+/* p ? a : b as one SEL: nvcc turns chains of ?: between lane-dependent values into divergent branches */
+__device__ __forceinline__ float sel(bool p, float a, float b) {
+  float r;
+  asm("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %3, 0;\n\tselp.f32 %0, %1, %2, q;\n\t}" : "=f"(r) : "f"(a), "f"(b), "r"((unsigned)p));
+  return r;
+}
+template <int K>
+__device__ __forceinline__ float xch_pick(unsigned m, const float* v) {
+  return sel(m == 3u, v[3], sel(m == 0u, v[0], v[1 + (K & 1)]));
+}
+/* foot layout (pgs_lane_init4) -> sweep layout, bit for bit; column by column, so that the two copies of B are
+ * not live at once */
+__device__ __forceinline__ void pgs_rows_exchange4(const PgsLane4& pl, int leg, unsigned gbase, PgsRows4& pr) {
+  const unsigned kFull = 0xffffffffu;
+  unsigned src[4], m[4];
+#pragma unroll
+  for (int k = 0; k < 4; k++) { src[k] = gbase + xch_field(kXchSrc, k, leg); m[k] = xch_field(kXchRow, k, leg); }
+#pragma unroll
+  for (int c = 0; c < kRowsL + 2; c++) {
+    float v[4];
+#pragma unroll
+    for (int r = 0; r < 4; r++) v[r] = (c < kRowsL) ? pl.B[r][c] : (c == kRowsL ? pl.g[r] : pl.diag[r]);
+    float w[4];
+    w[0] = __shfl_sync(kFull, xch_pick<0>(m[0], v), src[0]);
+    w[1] = __shfl_sync(kFull, xch_pick<1>(m[1], v), src[1]);
+    w[2] = __shfl_sync(kFull, xch_pick<2>(m[2], v), src[2]);
+    w[3] = __shfl_sync(kFull, xch_pick<3>(m[3], v), src[3]);
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+      if (c < kRowsL) pr.B[k][c] = w[k];
+      else if (c == kRowsL) pr.g[k] = w[k];
+      else pr.diag[k] = w[k];
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < 4; k++) pr.x[k] = 0.f;
+}
+/* round K of the way back: this lane's impulse of row m = kXchRow[K][leg]; lam4 = {normal, friction A, B, limit} */
+template <int K>
+__device__ __forceinline__ void xch_back_round(const float* lam_slot, int leg, unsigned gbase, float* lam4) {
+  const float v = __shfl_sync(0xffffffffu, lam_slot[K], gbase + xch_field(kXchDst, K, leg));
+  const unsigned m = xch_field(kXchRow, K, leg);
+  lam4[0] = sel(m == 0u, v, lam4[0]);
+  lam4[1 + (K & 1)] = sel(m == 1u + (K & 1), v, lam4[1 + (K & 1)]);
+  lam4[3] = sel(m == 3u, v, lam4[3]);
+}
+
+/* rows g[2P], g[2P+1] += B[.][col] * d (B stored negated) */
+__device__ __forceinline__ void pair_apply(const PgsRows4& pr, float* g, int P, int col, float d) {
+  pgs_fma_pair(g[2 * P], g[2 * P + 1], pr.B[2 * P][col], pr.B[2 * P + 1][col], d);
+}
+/* the owner's scratch rows t after change i of a phase: only the pairs a later relaxation of the phase reads
+ * (last[P] = position in the phase of pair P's last relaxation) */
+__device__ __forceinline__ void phase_scratch_apply(const PgsRows4& pr, float* t, int i, int col, float d,
+                                                    const int* last) {
+#pragma unroll
+  for (int P = 0; P < 2; P++)
+    if (i < last[P]) pair_apply(pr, t, P, col, d);
+}
+/* the hand-over: the phase's four changes, shuffled from its owner, to the rows of every lane */
+__device__ __forceinline__ void phase_hand_over(PgsRows4& pr, const int* cols, const float* d) {
+#pragma unroll
+  for (int P = 0; P < 2; P++) {
+#pragma unroll
+    for (int i = 0; i < 4; i++) pair_apply(pr, pr.g, P, cols[i], d[i]);
+  }
+}
+
+/* the friction pairs of feet fb, fb + 1 (fb = 2 (o - 2)) on lane o; returns the largest |residual| of the phase */
+template <bool CONE>
+__device__ __forceinline__ float friction_phase4(PgsRows4& pr, int leg, unsigned gbase, int o, const float* nvN,
+                                                 float mu) {
+  const unsigned kFull = 0xffffffffu;
+  const bool own = (leg == o);
+  const int fb = 2 * (o - 2);
+  const int last[2] = {CONE ? 0 : 1, CONE ? 2 : 3};   /* a cone pair takes both candidates from one state */
+  float t[4] = {pr.g[0], pr.g[1], pr.g[2], pr.g[3]};
+  float res = 0.f;
+  int cols[4];
+  float d[4];
+#pragma unroll
+  for (int i = 0; i < 4; i++) cols[i] = row_of(fb, 1) + i;
+#pragma unroll
+  for (int p = 0; p < 2; p++) {
+    const int a = 2 * p, b = 2 * p + 1;
+    if (CONE) {
+      float nA, nB, dA, dB, rv;
+      cone_candidate(mu, nvN[fb + p], t[a], t[b], pr.x[a], pr.x[b], pr.diag[a], pr.diag[b], nA, nB, dA, dB, rv);
+      d[a] = __shfl_sync(kFull, dA, gbase + o);
+      d[b] = __shfl_sync(kFull, dB, gbase + o);
+      if (own) { pr.x[a] = nA; pr.x[b] = nB; }
+      res = fmaxf(res, fabsf(rv));
+      phase_scratch_apply(pr, t, a, cols[a], dA, last);
+      phase_scratch_apply(pr, t, b, cols[b], dB, last);
+    } else {
+#pragma unroll
+      for (int q = 0; q < 2; q++) {
+        const int s = a + q;
+        float nv, dq, rv;
+        pyramid_candidate(mu, nvN[fb + p], t[s], pr.x[s], pr.diag[s], nv, dq, rv);
+        d[s] = __shfl_sync(kFull, dq, gbase + o);
+        if (own) pr.x[s] = nv;
+        res = fmaxf(res, fabsf(rv));
+        phase_scratch_apply(pr, t, s, cols[s], dq, last);
+      }
+    }
+  }
+  phase_hand_over(pr, cols, d);
+  return res;
+}
+
+template <bool CONE>
+__device__ __forceinline__ void pgs_sweeps4_phased(PgsRows4& pr, const SimConst& sc, int leg, unsigned gbase, unsigned amask,
+                                            unsigned lmask, int nc, float* lam4, int& sweep_feet, const EnvDyn* dyn) {
+  const unsigned kFull = 0xffffffffu;
+  const float mu = env_mu(sc, dyn);
+  bool conv = (amask == 0) && (lmask == 0);
+  /* the impulses of the sweep that converged; lanes 0 and 1 latch -lambda (-0 stands for an impulse of +0) */
+  float held[4];
+#pragma unroll
+  for (int s = 0; s < 4; s++) held[s] = sel(leg < 2, -0.f, 0.f);
+  for (int it = 0; it < sc.iters; it++) {
+    sweep_feet += conv ? 0 : nc;
+    /* Each phase's residual is taken on every lane and the owner's kept at the end: the exit test only asks whether
+     * the largest residual of the env's sweep is within the threshold, whichever lane holds it. */
+    float resL = 0.f, resN = 0.f;
+    {   /* (a warp-uniform `if (lwarp)` around this block was measured slower: 94.6 vs 90.1 us at 4096 envs) */
+      /* the (at most four) limit rows of an env belong to different legs and are relaxed as ONE group: every
+       * candidate is taken from the same state.  With a single limit row per env (99.5 % of the cases under random
+       * actions) this IS Bullet's sequential order; with several it is a Jacobi step among rows that couple only
+       * through the base.  h-rows (PgsLaneT): lambda + d = min(max(candidate, 0), max_impulse). */
+      const bool own = (leg == 0);
+      float d[4];
+      int cols[4];
+#pragma unroll
+      for (int s = 0; s < 4; s++) {
+        const float ul = sc.lim_max_impulse + pr.x[s];
+        const float dl = fminf(fmaxf(pr.g[s], pr.x[s]), ul);
+        const float nv = dl - pr.x[s];
+        resL = fmaxf(resL, fabsf(dl * pr.diag[s]));
+        if (own) pr.x[s] = -nv;
+        d[kLimLeg[s]] = __shfl_sync(kFull, dl, gbase + 0);
+      }
+#pragma unroll
+      for (int j = 0; j < 4; j++) cols[j] = limit_col(j);
+      phase_hand_over(pr, cols, d);
+    }
+    float nvN[4];
+    {   /* the normal rows, foot by foot; h-rows: lambda + d = max(candidate, 0) */
+      const bool own = (leg == 1);
+      const int last[2] = {3, 2};   /* the highest foot of each pair: slots 0, 1 hold feet 3, 1; slots 2, 3 feet 2, 0 */
+      float t[4] = {pr.g[0], pr.g[1], pr.g[2], pr.g[3]};
+      float d[4];
+      int cols[4];
+#pragma unroll
+      for (int f = 0; f < 4; f++) {
+        const int s = kNrmFoot[f];
+        const float dn = fmaxf(t[s], pr.x[s]);
+        const float nv = dn - pr.x[s];
+        resN = fmaxf(resN, fabsf(dn * pr.diag[s]));
+        d[f] = __shfl_sync(kFull, dn, gbase + 1);
+        nvN[f] = __shfl_sync(kFull, nv, gbase + 1);
+        if (own) pr.x[s] = -nv;
+        cols[f] = row_of(f, 0);
+        phase_scratch_apply(pr, t, f, cols[f], dn, last);
+      }
+      phase_hand_over(pr, cols, d);
+    }
+    const float resF0 = friction_phase4<CONE>(pr, leg, gbase, 2, nvN, mu);
+    const float resF1 = friction_phase4<CONE>(pr, leg, gbase, 3, nvN, mu);
+    const float res_own = sel(leg < 2, sel(leg == 0, resL, resN), sel(leg == 2, resF0, resF1));
+    if (!conv) {
+#pragma unroll
+      for (int s = 0; s < 4; s++) held[s] = pr.x[s];
+    }
+    /* end of sweep, Bullet's exit test: the env is done when every row residual of the sweep is within the
+     * threshold, i.e. when each of its four lanes is; one ballot serves the env test and the warp-wide loop exit */
+    const unsigned okb = __ballot_sync(kFull, conv || (res_own * res_own <= sc.res_thr));
+    conv = conv || (((okb >> gbase) & 0xFu) == 0xFu);
+    if (okb == kFull) break;
+  }
+  float lam_slot[4];
+#pragma unroll
+  for (int s = 0; s < 4; s++) lam_slot[s] = sel(leg < 2, -held[s], held[s]);
+  lam4[0] = lam4[1] = lam4[2] = lam4[3] = 0.f;
+  xch_back_round<0>(lam_slot, leg, gbase, lam4);
+  xch_back_round<1>(lam_slot, leg, gbase, lam4);
+  xch_back_round<2>(lam_slot, leg, gbase, lam4);
+  xch_back_round<3>(lam_slot, leg, gbase, lam4);
+}
+
 /* SOLO_TRACE builds (tools only): cycle stamps inside the substeps of the narrow builds, lane 0 of every block */
 #ifdef SOLO_TRACE
 __device__ long long g_narrow_trace[1024][8][8];
@@ -446,7 +673,7 @@ __device__ int g_trace_substep;
 /* Second half of a substep for the four lanes of an env: contact / joint-limit rows -> Delassus rows ->
  * projected Gauss-Seidel -> impulses -> position update.  In: ln (P, K, sP, Lm, b, dist, active of the own
  * foot and the ABA by-products r, ax, h, invD), bw (pre-update rotation, LDL factor), the limit-row selection. */
-template <int NJL, bool LIMITS, bool BODY>
+template <int NJL, bool LIMITS, bool BODY, bool PHASED = false>
 __device__ __forceinline__ void contact_solve(const SimConst& sc, int leg, BaseState& st, const BaseWork& bw,
                                               Lane<NJL>& ln, bool lim_env, int kL, float dirL, float penL,
                                               float& cforce, int& nc_sum, int& sweep_feet, int g_trace_sub = 0,
@@ -488,6 +715,7 @@ __device__ __forceinline__ void contact_solve(const SimConst& sc, int leg, BaseS
     LimitRow<NJL> lr;
     limit_setup<NJL>(sc, bw, ln, lim_any, kL, dirL, penL, lr);
     PgsLane4 pl;
+    PgsRows4 pr;   /* PHASED: the sweep layout of pgs_sweeps4_phased */
     {
       float rows[4][kRowsL];
 #pragma unroll
@@ -504,13 +732,19 @@ __device__ __forceinline__ void contact_solve(const SimConst& sc, int leg, BaseS
         assemble_block4<NJL>(ln, lr, leg, j, Kj, KLj, col_on, rows);
       }
       pgs_lane_init4<NJL>(ln, lr, leg, rows, amask, lmask, sc.lim_max_impulse, pl);
+      if (PHASED) pgs_rows_exchange4(pl, leg, gbase, pr);
     }
     const int nc = __popc(amask);
     nc_sum += nc;
     float lam4[4];
     NSTAMP(3);
-    if (sc.cone) pgs_sweeps4<true>(pl, sc, leg, gbase, amask, lmask, lwarp, nc, lam4, sweep_feet, dyn);
-    else pgs_sweeps4<false>(pl, sc, leg, gbase, amask, lmask, lwarp, nc, lam4, sweep_feet, dyn);
+    if (PHASED) {
+      if (sc.cone) pgs_sweeps4_phased<true>(pr, sc, leg, gbase, amask, lmask, nc, lam4, sweep_feet, dyn);
+      else pgs_sweeps4_phased<false>(pr, sc, leg, gbase, amask, lmask, nc, lam4, sweep_feet, dyn);
+    } else {
+      if (sc.cone) pgs_sweeps4<true>(pl, sc, leg, gbase, amask, lmask, lwarp, nc, lam4, sweep_feet, dyn);
+      else pgs_sweeps4<false>(pl, sc, leg, gbase, amask, lmask, lwarp, nc, lam4, sweep_feet, dyn);
+    }
     NSTAMP(4);
     lam3[0] = lam4[0]; lam3[1] = lam4[1]; lam3[2] = lam4[2];
     float part[6], dv0[6];
@@ -588,7 +822,7 @@ __device__ __forceinline__ void contact_solve(const SimConst& sc, int leg, BaseS
  * Control flow is kept WARP-uniform (skip masks and the sweep-loop exit are warp votes, envs that
  * have nothing to do contribute exact zeros) so that every shuffle is a full-mask shuffle of a
  * converged warp: group-masked shuffles cost a WARPSYNC each and let the 4-lane groups drift apart. */
-template <int NJL, bool LIMITS, bool BODY = false>
+template <int NJL, bool LIMITS, bool BODY = false, bool PHASED = false>
 __device__ __forceinline__ void group_substep(const LegConst& lc, const ModelConst& mc, const SimConst& sc,
                                               int leg, BaseState& st, Lane<NJL>& ln, const float* tau, float& cforce,
                                               int& nc_sum, int& sweep_feet, int g_trace_sub = 0,
@@ -623,7 +857,7 @@ __device__ __forceinline__ void group_substep(const LegConst& lc, const ModelCon
   int kL;
   float dirL, penL;
   const bool lim_any = LIMITS && limit_select<NJL>(sc, ln, kL, dirL, penL);
-  contact_solve<NJL, LIMITS, BODY>(sc, leg, st, bw, ln, lim_any, kL, dirL, penL, cforce, nc_sum, sweep_feet, g_trace_sub,
+  contact_solve<NJL, LIMITS, BODY, PHASED>(sc, leg, st, bw, ln, lim_any, kL, dirL, penL, cforce, nc_sum, sweep_feet, g_trace_sub,
                                    body_rows, dyn);
   NSTAMP(5);
 }
@@ -849,8 +1083,14 @@ __device__ __forceinline__ void step_finish(const StepArgs& args, int wslot, Sta
  * builds without it are the code of a handle that has never heard of randomisation.
  * PUSH (SoloSimParams.push_interval > 0), instantiated with RAND only: step_load puts the env's push for the
  * launch into the warp's stage, and every substep reads it from there as the external force on the base; a handle
- * with pushes and without randomisation passes envp == nullptr and runs the nominal dynamics. */
-template <int NJL, int MINB, int WPB, bool LIMITS, bool BODY = false, bool RAND = false, bool PUSH = false>
+ * with pushes and without randomisation passes envp == nullptr and runs the nominal dynamics.
+ * PHASED: the four-row sweep with the rows placed by sweep position (pgs_sweeps4_phased), for the latency build,
+ * whose launch is one resident wave and so lasts as long as its slowest env's sweep chain.  The throughput build,
+ * bound by issue slots at several resident waves, keeps pgs_sweeps4 (same bits, fewer instructions), and so does the
+ * body build, whose step is set by the general path's sweeps (measured: -0.7 % to +1.1 % per step with the phased
+ * sweep, and more spills in the solo8 +rand+push instantiation). */
+template <int NJL, int MINB, int WPB, bool LIMITS, bool BODY = false, bool RAND = false, bool PUSH = false,
+          bool PHASED = false>
 __global__ void __launch_bounds__(kBlockThreads * WPB, MINB) step_kernel(const __grid_constant__ StepArgs args,
                                                                          const __grid_constant__ DynArgs dyn) {
   __shared__ Smem sm;
@@ -878,8 +1118,8 @@ __global__ void __launch_bounds__(kBlockThreads * WPB, MINB) step_kernel(const _
     float tau_s[NJL];
 #pragma unroll
     for (int k = 0; k < NJL; k++) tau_s[k] = torque_on ? L.tau[k] : 0.f;
-    group_substep<NJL, LIMITS, BODY>(sm.leg[L.leg], args.mc, sc, L.leg, L.st, L.ln, tau_s, L.cforce, L.bk.nc_sum,
-                                     L.bk.sweep_feet, s, PUSH ? &stage[wib][L.el][0] : nullptr,
+    group_substep<NJL, LIMITS, BODY, PHASED>(sm.leg[L.leg], args.mc, sc, L.leg, L.st, L.ln, tau_s, L.cforce,
+                                                L.bk.nc_sum, L.bk.sweep_feet, s, PUSH ? &stage[wib][L.el][0] : nullptr,
                                      BODY ? body_smem + (size_t)(wib * 8 + L.el) * kBodyEnvStride : nullptr,
                                      RAND ? &L.dyn : nullptr);
   }
@@ -978,7 +1218,8 @@ __global__ void __launch_bounds__(kBlockThreads) actuator_kernel(const __grid_co
 #pragma unroll
     for (int k = 0; k < NJL; k++) tau[k] = actuator_torque(sc, ln.q[k], ln.qd[k], qdes[k], vdes[k], P[k], D[k], tff[k]);
     float* const rows = BODY ? body_smem + (size_t)el * kBodyEnvStride : nullptr;
-    if (sc.joint_limits) group_substep<NJL, true, BODY>(sm.leg[leg], args.mc, sc, leg, st, ln, tau, cforce, nc_sum, sweep_feet, 0, fext, rows);
+    /* the phased sweep as in the latency build; with body contacts the foot layout, as in the body build */
+    if (sc.joint_limits) group_substep<NJL, true, BODY, !BODY>(sm.leg[leg], args.mc, sc, leg, st, ln, tau, cforce, nc_sum, sweep_feet, 0, fext, rows);
     else group_substep<NJL, false, BODY>(sm.leg[leg], args.mc, sc, leg, st, ln, tau, cforce, nc_sum, sweep_feet, 0, fext, rows);
   }
   if (valid) {
@@ -1473,18 +1714,18 @@ static DynArgs dyn_args(const SoloHandle* h) {
   if (!h->randomize) a.envp = nullptr;
   return a;
 }
-template <int MINB, int WPB, bool RAND, bool PUSH = false>
+template <int MINB, int WPB, bool PHASED, bool RAND, bool PUSH = false>
 static void launch_step_variant(SoloHandle* h, const StepArgs& a, cudaStream_t s) {
   int blocks = (a.n + 8 * WPB - 1) / (8 * WPB);
   if (blocks < grid_min()) blocks = grid_min();
   const bool lim = h->sc.joint_limits != 0;
   const DynArgs dyn = dyn_args(h);
   if (h->njl == 3) {
-    if (lim) step_kernel<3, MINB, WPB, true, false, RAND, PUSH><<<blocks, kBlockThreads * WPB, 0, s>>>(a, dyn);
-    else step_kernel<3, MINB, WPB, false, false, RAND, PUSH><<<blocks, kBlockThreads * WPB, 0, s>>>(a, dyn);
+    if (lim) step_kernel<3, MINB, WPB, true, false, RAND, PUSH, PHASED><<<blocks, kBlockThreads * WPB, 0, s>>>(a, dyn);
+    else step_kernel<3, MINB, WPB, false, false, RAND, PUSH, PHASED><<<blocks, kBlockThreads * WPB, 0, s>>>(a, dyn);
   } else {
-    if (lim) step_kernel<2, MINB, WPB, true, false, RAND, PUSH><<<blocks, kBlockThreads * WPB, 0, s>>>(a, dyn);
-    else step_kernel<2, MINB, WPB, false, false, RAND, PUSH><<<blocks, kBlockThreads * WPB, 0, s>>>(a, dyn);
+    if (lim) step_kernel<2, MINB, WPB, true, false, RAND, PUSH, PHASED><<<blocks, kBlockThreads * WPB, 0, s>>>(a, dyn);
+    else step_kernel<2, MINB, WPB, false, false, RAND, PUSH, PHASED><<<blocks, kBlockThreads * WPB, 0, s>>>(a, dyn);
   }
 }
 /* shape of the throughput build: warps per block and resident blocks per SM (the register cap follows:
@@ -1533,13 +1774,13 @@ static void launch_step(SoloHandle* h, const StepArgs& a, cudaStream_t s) {
       else wide_step_kernel<2, false><<<blocks, kWThreads, sizeof(WideShared), s>>>(a);
     }
   } else if (h->variant == VARIANT_THROUGHPUT) {
-    if (h->push) launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB, true, true>(h, a, s);
-    else if (h->randomize) launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB, true>(h, a, s);
-    else launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB, false>(h, a, s);
+    if (h->push) launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB, false, true, true>(h, a, s);
+    else if (h->randomize) launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB, false, true>(h, a, s);
+    else launch_step_variant<SOLO_TP_MINB, SOLO_TP_WPB, false, false>(h, a, s);
   } else {
-    if (h->push) launch_step_variant<1, 4, true, true>(h, a, s);
-    else if (h->randomize) launch_step_variant<1, 4, true>(h, a, s);
-    else launch_step_variant<1, 4, false>(h, a, s);
+    if (h->push) launch_step_variant<1, 4, true, true, true>(h, a, s);
+    else if (h->randomize) launch_step_variant<1, 4, true, true>(h, a, s);
+    else launch_step_variant<1, 4, true, false>(h, a, s);
   }
   h->launches++;
 }
