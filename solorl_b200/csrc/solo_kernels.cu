@@ -446,12 +446,13 @@ __device__ __forceinline__ void pgs_sweeps4(PgsLane4& pl, const SimConst& sc, in
  * one lane per foot (pgs_sweeps4), and the result is bit-identical to it.  The slot orders of lanes 0 and 1 follow
  * from the exchange schedule of pgs_rows_exchange4.
  * It issues more instructions per sweep than pgs_sweeps4 (limit candidates on one lane, the owner's scratch FMAs, the
- * normal impulses sent to the friction lanes) for a shorter chain: faster where one env's chain bounds the launch
+ * impulse updates of every phase on every lane) for a shorter chain: faster where one env's chain bounds the launch
  * (latency build, 4096 envs), slower where issue slots do (throughput build, 65 536 envs); see PHASED of step_kernel. */
 struct PgsRows4 {
   float B[4][kRowsL];   /* negated, scaled Delassus rows (PgsLaneT) */
   float g[4], diag[4];
-  float x[4];           /* -lambda on lanes 0 and 1 (the h-rows' lower bound of the impulse change), lambda on 2, 3 */
+  float x[4];           /* lambda of the limit rows on lane 0, of the friction rows on lanes 2, 3 (set by the sweep;
+                         * the normal impulses are held by every lane of the env, in the sweep's lamN) */
 };
 __device__ constexpr int kLimLeg[4] = {1, 3, 0, 2};
 __device__ constexpr int kNrmFoot[4] = {3, 1, 2, 0};   /* its own inverse */
@@ -472,6 +473,17 @@ __device__ __forceinline__ float sel(bool p, float a, float b) {
   float r;
   asm("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %3, 0;\n\tselp.f32 %0, %1, %2, q;\n\t}" : "=f"(r) : "f"(a), "f"(b), "r"((unsigned)p));
   return r;
+}
+/* v of lane o of this lane's env: the lane as an immediate of the shuffle (segments of 4 lanes), no register for it */
+template <int O>
+__device__ __forceinline__ float shfl_env(float v) {
+  float r;
+  asm("shfl.sync.idx.b32 %0, %1, %2, 0x1c1f, 0xffffffff;" : "=f"(r) : "f"(v), "n"(O));
+  return r;
+}
+/* a += b where p, as one predicated add */
+__device__ __forceinline__ void add_if(bool p, int& a, int b) {
+  asm("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %1, 0;\n\t@q add.s32 %0, %0, %2;\n\t}" : "+r"(a) : "r"((unsigned)p), "r"(b));
 }
 template <int K>
 __device__ __forceinline__ float xch_pick(unsigned m, const float* v) {
@@ -501,13 +513,12 @@ __device__ __forceinline__ void pgs_rows_exchange4(const PgsLane4& pl, int leg, 
       else pr.diag[k] = w[k];
     }
   }
-#pragma unroll
-  for (int k = 0; k < 4; k++) pr.x[k] = 0.f;
 }
 /* round K of the way back: this lane's impulse of row m = kXchRow[K][leg]; lam4 = {normal, friction A, B, limit} */
 template <int K>
-__device__ __forceinline__ void xch_back_round(const float* lam_slot, int leg, unsigned gbase, float* lam4) {
-  const float v = __shfl_sync(0xffffffffu, lam_slot[K], gbase + xch_field(kXchDst, K, leg));
+__device__ __forceinline__ void xch_back_round(const float* lam_slot, int leg, float* lam4) {
+  float v;
+  asm("shfl.sync.idx.b32 %0, %1, %2, 0x1c1f, 0xffffffff;" : "=f"(v) : "f"(lam_slot[K]), "r"(xch_field(kXchDst, K, leg)));
   const unsigned m = xch_field(kXchRow, K, leg);
   lam4[0] = sel(m == 0u, v, lam4[0]);
   lam4[1 + (K & 1)] = sel(m == 1u + (K & 1), v, lam4[1 + (K & 1)]);
@@ -535,13 +546,11 @@ __device__ __forceinline__ void phase_hand_over(PgsRows4& pr, const int* cols, c
   }
 }
 
-/* the friction pairs of feet fb, fb + 1 (fb = 2 (o - 2)) on lane o; returns the largest |residual| of the phase */
-template <bool CONE>
-__device__ __forceinline__ float friction_phase4(PgsRows4& pr, int leg, unsigned gbase, int o, const float* nvN,
-                                                 float mu) {
-  const unsigned kFull = 0xffffffffu;
-  const bool own = (leg == o);
-  const int fb = 2 * (o - 2);
+/* the friction pairs of feet fb, fb + 1 (fb = 2 (O - 2)) on lane O (own: this lane is O and its env still sweeps);
+ * lamN = the normal impulses; returns the largest |residual| of the phase */
+template <bool CONE, int O>
+__device__ __forceinline__ float friction_phase4(PgsRows4& pr, bool own, const float* lamN, float mu) {
+  const int fb = 2 * (O - 2);
   const int last[2] = {CONE ? 0 : 1, CONE ? 2 : 3};   /* a cone pair takes both candidates from one state */
   float t[4] = {pr.g[0], pr.g[1], pr.g[2], pr.g[3]};
   float res = 0.f;
@@ -554,9 +563,9 @@ __device__ __forceinline__ float friction_phase4(PgsRows4& pr, int leg, unsigned
     const int a = 2 * p, b = 2 * p + 1;
     if (CONE) {
       float nA, nB, dA, dB, rv;
-      cone_candidate(mu, nvN[fb + p], t[a], t[b], pr.x[a], pr.x[b], pr.diag[a], pr.diag[b], nA, nB, dA, dB, rv);
-      d[a] = __shfl_sync(kFull, dA, gbase + o);
-      d[b] = __shfl_sync(kFull, dB, gbase + o);
+      cone_candidate(mu, lamN[fb + p], t[a], t[b], pr.x[a], pr.x[b], pr.diag[a], pr.diag[b], nA, nB, dA, dB, rv);
+      d[a] = shfl_env<O>(dA);
+      d[b] = shfl_env<O>(dB);
       if (own) { pr.x[a] = nA; pr.x[b] = nB; }
       res = fmaxf(res, fabsf(rv));
       phase_scratch_apply(pr, t, a, cols[a], dA, last);
@@ -566,8 +575,8 @@ __device__ __forceinline__ float friction_phase4(PgsRows4& pr, int leg, unsigned
       for (int q = 0; q < 2; q++) {
         const int s = a + q;
         float nv, dq, rv;
-        pyramid_candidate(mu, nvN[fb + p], t[s], pr.x[s], pr.diag[s], nv, dq, rv);
-        d[s] = __shfl_sync(kFull, dq, gbase + o);
+        pyramid_candidate(mu, lamN[fb + p], t[s], pr.x[s], pr.diag[s], nv, dq, rv);
+        d[s] = shfl_env<O>(dq);
         if (own) pr.x[s] = nv;
         res = fmaxf(res, fabsf(rv));
         phase_scratch_apply(pr, t, s, cols[s], dq, last);
@@ -578,45 +587,50 @@ __device__ __forceinline__ float friction_phase4(PgsRows4& pr, int leg, unsigned
   return res;
 }
 
+/* The impulses.  Lane 0 keeps those of its limit rows and lanes 2, 3 those of their friction rows in x; the normal
+ * impulses are kept by every lane of the env (lamN, by foot), each updated from the shuffled change, so that the
+ * friction lanes read them without a shuffle of their own and lane 1 needs no select.  lambda + d is the same sum, in
+ * the same bits, as the h-row's d - (-lambda).  An env that met the exit test stops writing its impulses (the
+ * predicates below), so that they hold the values of the sweep that converged: the env keeps relaxing until the whole
+ * warp is done, without a latch per sweep or any select on the chain. */
 template <bool CONE>
 __device__ __forceinline__ void pgs_sweeps4_phased(PgsRows4& pr, const SimConst& sc, int leg, unsigned gbase, unsigned amask,
                                             unsigned lmask, int nc, float* lam4, int& sweep_feet, const EnvDyn* dyn) {
   const unsigned kFull = 0xffffffffu;
   const float mu = env_mu(sc, dyn);
+  const float lim_max = sc.lim_max_impulse, res_thr = sc.res_thr;
+  const unsigned env_top = 28u - gbase;
   bool conv = (amask == 0) && (lmask == 0);
-  /* the impulses of the sweep that converged; lanes 0 and 1 latch -lambda (-0 stands for an impulse of +0) */
-  float held[4];
+  /* lambda = +0; sweeps start from -0, the negation of the -lambda = +0 of the h-rows (pgs_sweeps4) */
+  const float z = conv ? 0.f : -0.f;
+  float lamN[4];
 #pragma unroll
-  for (int s = 0; s < 4; s++) held[s] = sel(leg < 2, -0.f, 0.f);
+  for (int s = 0; s < 4; s++) { pr.x[s] = sel(leg == 0, z, 0.f); lamN[s] = z; }
   for (int it = 0; it < sc.iters; it++) {
-    sweep_feet += conv ? 0 : nc;
     /* Each phase's residual is taken on every lane and the owner's kept at the end: the exit test only asks whether
      * the largest residual of the env's sweep is within the threshold, whichever lane holds it. */
+    const int role = conv ? 4 : leg;   /* the phase whose impulses this lane writes; none once its env has converged */
     float resL = 0.f, resN = 0.f;
     {   /* (a warp-uniform `if (lwarp)` around this block was measured slower: 94.6 vs 90.1 us at 4096 envs) */
       /* the (at most four) limit rows of an env belong to different legs and are relaxed as ONE group: every
        * candidate is taken from the same state.  With a single limit row per env (99.5 % of the cases under random
        * actions) this IS Bullet's sequential order; with several it is a Jacobi step among rows that couple only
        * through the base.  h-rows (PgsLaneT): lambda + d = min(max(candidate, 0), max_impulse). */
-      const bool own = (leg == 0);
+      const bool own = (role == 0);
       float d[4];
       int cols[4];
 #pragma unroll
       for (int s = 0; s < 4; s++) {
-        const float ul = sc.lim_max_impulse + pr.x[s];
-        const float dl = fminf(fmaxf(pr.g[s], pr.x[s]), ul);
-        const float nv = dl - pr.x[s];
+        const float dl = fminf(fmaxf(pr.g[s], -pr.x[s]), lim_max - pr.x[s]);
         resL = fmaxf(resL, fabsf(dl * pr.diag[s]));
-        if (own) pr.x[s] = -nv;
-        d[kLimLeg[s]] = __shfl_sync(kFull, dl, gbase + 0);
+        if (own) pr.x[s] = dl + pr.x[s];
+        d[kLimLeg[s]] = shfl_env<0>(dl);
       }
 #pragma unroll
       for (int j = 0; j < 4; j++) cols[j] = limit_col(j);
       phase_hand_over(pr, cols, d);
     }
-    float nvN[4];
     {   /* the normal rows, foot by foot; h-rows: lambda + d = max(candidate, 0) */
-      const bool own = (leg == 1);
       const int last[2] = {3, 2};   /* the highest foot of each pair: slots 0, 1 hold feet 3, 1; slots 2, 3 feet 2, 0 */
       float t[4] = {pr.g[0], pr.g[1], pr.g[2], pr.g[3]};
       float d[4];
@@ -624,38 +638,37 @@ __device__ __forceinline__ void pgs_sweeps4_phased(PgsRows4& pr, const SimConst&
 #pragma unroll
       for (int f = 0; f < 4; f++) {
         const int s = kNrmFoot[f];
-        const float dn = fmaxf(t[s], pr.x[s]);
-        const float nv = dn - pr.x[s];
+        const float dn = fmaxf(t[s], -lamN[f]);
         resN = fmaxf(resN, fabsf(dn * pr.diag[s]));
-        d[f] = __shfl_sync(kFull, dn, gbase + 1);
-        nvN[f] = __shfl_sync(kFull, nv, gbase + 1);
-        if (own) pr.x[s] = -nv;
+        d[f] = shfl_env<1>(dn);
         cols[f] = row_of(f, 0);
         phase_scratch_apply(pr, t, f, cols[f], dn, last);
       }
       phase_hand_over(pr, cols, d);
-    }
-    const float resF0 = friction_phase4<CONE>(pr, leg, gbase, 2, nvN, mu);
-    const float resF1 = friction_phase4<CONE>(pr, leg, gbase, 3, nvN, mu);
-    const float res_own = sel(leg < 2, sel(leg == 0, resL, resN), sel(leg == 2, resF0, resF1));
-    if (!conv) {
+      if (!conv) {
 #pragma unroll
-      for (int s = 0; s < 4; s++) held[s] = pr.x[s];
+        for (int f = 0; f < 4; f++) lamN[f] = d[f] + lamN[f];
+      }
     }
+    const float resF0 = friction_phase4<CONE, 2>(pr, role == 2, lamN, mu);
+    const float resF1 = friction_phase4<CONE, 3>(pr, role == 3, lamN, mu);
+    /* (a converged env's residual is not looked at) */
+    const float res_own = sel(role < 2, sel(role == 0, resL, resN), sel(role == 2, resF0, resF1));
     /* end of sweep, Bullet's exit test: the env is done when every row residual of the sweep is within the
      * threshold, i.e. when each of its four lanes is; one ballot serves the env test and the warp-wide loop exit */
-    const unsigned okb = __ballot_sync(kFull, conv || (res_own * res_own <= sc.res_thr));
-    conv = conv || (((okb >> gbase) & 0xFu) == 0xFu);
+    const unsigned okb = __ballot_sync(kFull, conv || (res_own * res_own <= res_thr));
+    add_if(!conv, sweep_feet, nc);
+    conv = conv || ((okb << env_top) >= 0xF0000000u);   /* the env's four bits of okb, moved to the top, all set */
     if (okb == kFull) break;
   }
   float lam_slot[4];
 #pragma unroll
-  for (int s = 0; s < 4; s++) lam_slot[s] = sel(leg < 2, -held[s], held[s]);
+  for (int s = 0; s < 4; s++) lam_slot[s] = sel(leg == 1, lamN[kNrmFoot[s]], pr.x[s]);
   lam4[0] = lam4[1] = lam4[2] = lam4[3] = 0.f;
-  xch_back_round<0>(lam_slot, leg, gbase, lam4);
-  xch_back_round<1>(lam_slot, leg, gbase, lam4);
-  xch_back_round<2>(lam_slot, leg, gbase, lam4);
-  xch_back_round<3>(lam_slot, leg, gbase, lam4);
+  xch_back_round<0>(lam_slot, leg, lam4);
+  xch_back_round<1>(lam_slot, leg, lam4);
+  xch_back_round<2>(lam_slot, leg, lam4);
+  xch_back_round<3>(lam_slot, leg, lam4);
 }
 
 /* SOLO_TRACE builds (tools only): cycle stamps inside the substeps of the narrow builds, lane 0 of every block */
